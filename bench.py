@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the segment-reduction hot path (contract: see DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl own|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl own|reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input.  Default workload (BASELINE.json
 configs[1], the configuration the metric is quoted on): gather_weight_scatter, GCN aggregation on a
@@ -84,7 +84,7 @@ def measured_peak_gbs():
             return float(json.load(open(p))["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
         except Exception:
             pass
-    return 6650.0, "fallback (B200_PROFILING.md)"
+    return 6564.0, "measured on an NVIDIA B200 at 1000 W power limit: 4 GiB device copy, read + write bytes"
 
 
 class ClockSampler:
@@ -241,7 +241,7 @@ def run_reference(args):
     dev = "cuda" if torch.cuda.is_available() else "cpu"
     scale = 1.0 if dev == "cuda" else 1.0 / 16
     wk = build_workload(args.workload, dev, scale)
-    steps, warmup = max(1, min(args.steps, 5)), max(1, min(args.warmup, 2))
+    steps, warmup = args.steps, args.warmup
     obj, sec, frac = cpu_arm(wk, warmup, steps)
     assert obj["cores"] > 1 or (os.cpu_count() or 1) == 1, "the CPU arm must use every host core"
     cfg = config_of(wk, args.gpus)
@@ -383,12 +383,13 @@ def barrier(world):
     torch.cuda.synchronize()
 
 
-def time_runner(r, steps, warmup, sampler=None):
+def time_runner(r, steps, warmup, sampler=None, keep_output=False):
     """W warm-up steps, then exactly K steps between barrier + synchronize, CUDA events on the launching stream, max
     over ranks.  The main kernel's own duration comes from a SECOND loop of K steps with the library's profiling hook
     on (an event pair around every main-kernel launch): the timed loop itself carries no instrumentation -- an event
     record between the main kernel and its programmatically dependent fixup launch would serialise the two and cost
-    the small shapes several microseconds per step.  Returns (ms per step, main-kernel ms per step)."""
+    the small shapes several microseconds per step.  `keep_output`: r.timed_output = a copy of what the last timed step
+    wrote, taken before the second loop.  Returns (ms per step, main-kernel ms per step)."""
     import torch.distributed as dist
     abi = r.abi
     for _ in range(max(warmup, 3)):
@@ -420,6 +421,8 @@ def time_runner(r, steps, warmup, sampler=None):
     ev[1].record()
     barrier(r.world)
     total_ms = ev[0].elapsed_time(ev[1])
+    if keep_output:
+        r.timed_output = r.out.clone()
     abi.profile_enable(steps * r.calls_per_step)
     for _ in range(steps):
         r.step()
@@ -432,6 +435,29 @@ def time_runner(r, steps, warmup, sampler=None):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         total_ms, kmean = t.tolist()
     return total_ms / steps, kmean
+
+
+DUMP_BYTES = 32 << 20       # --dump-outputs writes the whole output up to this size, a sample of its rows beyond
+
+
+def dump_outputs(out, directory):
+    """Writes the output of the timed step to DIR/output.npy (float64 for fp64 outputs, float32 otherwise) so that two
+    builds can be compared output for output.  An output larger than DUMP_BYTES is written as a fixed, seeded sample of
+    its rows, in ascending order; their indices go to DIR/output_rows.npy (float64)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    host = torch.float64 if out.dtype == torch.float64 else torch.float32
+    S = out.shape[0]
+    row_bytes = max(1, out.numel() // max(S, 1)) * torch.tensor([], dtype=host).element_size()
+    k = min(S, max(1, DUMP_BYTES // row_bytes))
+    rows_path = os.path.join(directory, "output_rows.npy")
+    if k < S:
+        rows = torch.randperm(S, generator=torch.Generator().manual_seed(0))[:k].sort().values
+        np.save(rows_path, rows.double().numpy())
+        out = out.index_select(0, rows.to(out.device))
+    elif os.path.exists(rows_path):
+        os.remove(rows_path)
+    np.save(os.path.join(directory, "output.npy"), out.to(host).cpu().numpy())
 
 
 def parity_check(r, rows_k=40):
@@ -553,7 +579,7 @@ def run_secondary(name, world, rank, dev, exchanges, steps, warmup, peak, with_c
             d["src_rows_received_per_step_rank0"], d["src_rows_full_exchange_rank0"] = r.exchanged
         d["shard_imbalance"] = round(r.imbalance, 4)
         if with_cpu and rank == 0:
-            d["cpu_baseline"], _, _ = cpu_arm(wk, 1, 3)
+            d["cpu_baseline"], _, _ = cpu_arm(wk, warmup, steps)
         res[exchange] = d
         del r
         torch.cuda.empty_cache()
@@ -654,10 +680,10 @@ def e2e_single(r, wk, n_e2e):
     st_call()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    for _ in range(3):
+    for _ in range(n_e2e):
         st_call()
     torch.cuda.synchronize()
-    st_s = (time.perf_counter() - t0) / 3
+    st_s = (time.perf_counter() - t0) / n_e2e
     st_h2d, st_d2h = abi.host_last_transfer()
     abi.lib().geot_b200_host_arena_release()
     return {"value": round(wk["bytes_logical"] / e2e_s / 1e9, 2), "unit": "GB/s", "h2d_bytes_per_step": h2d,
@@ -690,8 +716,14 @@ def run_own(args):
     wk = build_workload(args.workload, dev)
     r = Runner(wk, world, rank, dev, exchange)
     sampler = ClockSampler(local) if rank == 0 else None
-    ms_per_step, kmean = time_runner(r, args.steps, args.warmup, sampler)
+    ms_per_step, kmean = time_runner(r, args.steps, args.warmup, sampler, keep_output=bool(args.dump_outputs))
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # N > 1: each rank holds the output rows of its shard; rank 0 writes them assembled
+        out = r.timed_output if world == 1 else r.gdist.all_gather_rows(r.timed_output, r.shard.row_bounds)
+        if rank == 0:
+            dump_outputs(out, args.dump_outputs)
+        del r.timed_output, out
     value = wk["bytes_logical"] / (ms_per_step * 1e-3) / 1e9
     parity = parity_check(r)
 
@@ -720,7 +752,7 @@ def run_own(args):
     meta = dict(metric=metric_name(wk), dtype=DTYPE_NAME[wk["dtype"]], config=cfg, E=wk["E"],
                 launches=r.launches_per_step, exchange=r.exchange, imbalance=r.imbalance, exchanged=r.exchanged)
 
-    n_e2e = max(3, min(args.steps, 5))
+    n_e2e = args.steps
     cpu_obj = None
     if world > 1:
         e2e = e2e_multi(r, wk, world, rank, dev, n_e2e)
@@ -730,18 +762,17 @@ def run_own(args):
                            "(stderr); this repeats the device-resident value"}
     else:
         e2e = e2e_single(r, wk, n_e2e)
-        cpu_obj, _, _ = cpu_arm(wk, 1, 3)
+        cpu_obj, _, _ = cpu_arm(wk, args.warmup, args.steps)
     del r, wk
     torch.cuda.empty_cache()
 
     # ---- the other BASELINE configurations (every rank takes part at N > 1) ---------------------------------------
     secondary = {}
-    sec_steps = max(3, min(args.steps, 20))
     if args.workload == "reddit_gws" and os.environ.get("GEOT_B200_BENCH_SECONDARY", "1") == "1":
         if world > 1:
             other = "push" if exchange != "push" else "bucket"
             for name in ("products_gs64", "products_gs256"):
-                got = run_secondary(name, world, rank, dev, [exchange, other, "replicated"], sec_steps, args.warmup, peak)
+                got = run_secondary(name, world, rank, dev, [exchange, other, "replicated"], args.steps, args.warmup, peak)
                 secondary[name] = {
                     "inclusive": got[exchange], "inclusive_alt": got[other], "replicated": got["replicated"],
                     "note": "strong scaling of BASELINE configs[2]; `inclusive` moves the src rows inside the step with the "
@@ -751,7 +782,7 @@ def run_own(args):
             for name, cpu in (("reddit_index_scatter", False), ("config1_index_scatter", True), ("products_gs64", False),
                               ("products_gs64_gaps", False), ("products_gs256", False), ("arxiv_mh_spmm", False)):
                 try:
-                    secondary[name] = run_secondary(name, 1, 0, dev, ["none"], sec_steps, args.warmup, peak, with_cpu=cpu)["none"]
+                    secondary[name] = run_secondary(name, 1, 0, dev, ["none"], args.steps, args.warmup, peak, with_cpu=cpu)["none"]
                 except Exception as ex:       # a secondary line must not cost the headline
                     secondary[name] = {"error": repr(ex)}
                     torch.cuda.empty_cache()
@@ -787,11 +818,19 @@ def run_own(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of every timed loop: each workload on the GPU, the "
+                    "host-buffer (e2e) legs and the CPU baselines")
+    ap.add_argument("--warmup", type=int, default=5, help="untimed steps before each timed loop (at least 3 on the GPU)")
     ap.add_argument("--impl", default="own", choices=["own", "reference"])
     ap.add_argument("--workload", default="reddit_gws", choices=sorted(WORKLOADS))
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output of the last timed step to DIR/output.npy (see dump_outputs); with N > 1 "
+                         "GPUs rank 0 writes the output assembled from every rank's rows")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "own":
+        ap.error("--dump-outputs applies to --impl own")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -106,10 +106,11 @@ def install(rank=0, world=1):
     abi.lib = lambda: types.SimpleNamespace(geot_b200_workspace_bytes=lambda *a: 256, geot_b200_host_arena_release=lambda: 0)
 
 
-def run_own(workload, world=1, steps=2, warmup=3):
+def run_own(workload, world=1, steps=2, warmup=3, dump_outputs=None):
     """bench.run_own under the emulation; returns rank 0's JSON line (None on the other ranks)."""
     import bench
-    args = types.SimpleNamespace(gpus=world, steps=steps, warmup=warmup, impl="own", workload=workload)
+    args = types.SimpleNamespace(gpus=world, steps=steps, warmup=warmup, impl="own", workload=workload,
+                                 dump_outputs=dump_outputs)
     buf = io.StringIO()
     with contextlib.redirect_stdout(buf):
         bench.run_own(args)
@@ -117,10 +118,10 @@ def run_own(workload, world=1, steps=2, warmup=3):
     return json.loads(out.splitlines()[-1]) if out else None
 
 
-def worker(rank, world, port, exchange, workload, q):
+def worker(rank, world, port, exchange, workload, q, dump_outputs=None):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
                       LOCAL_RANK=str(rank), GEOT_B200_EXCHANGE=exchange)
     install(rank, world)
-    line = run_own(workload, world)
+    line = run_own(workload, world, dump_outputs=dump_outputs)
     if rank == 0:
         q.put(line)

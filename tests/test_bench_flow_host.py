@@ -7,6 +7,7 @@ import subprocess
 import sys
 
 import pytest
+import torch
 import torch.multiprocessing as mp
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -34,16 +35,47 @@ def test_single_gpu_line_contract():
     assert "workload" in line["config"] and line["gpu_launches"] > 0
 
 
+def _timed_output(workload):
+    """What the timed step computes on `workload`'s seeded inputs under the emulation (the oracle plays the kernels)."""
+    import bench
+    import oracle
+    wk = bench.build_workload(workload, "cpu")
+    return wk, oracle.segment_reduce(wk["x"], wk["si"], wk["di"], wk["w"], "sum", S=wk["S"], H=wk["H"])
+
+
+def test_dump_outputs(tmp_path):
+    """--dump-outputs: the timed step's output as float32 .npy, whole or as a seeded sample of rows, the same from run to
+    run."""
+    import numpy as np
+    whole, sampled = str(tmp_path / "whole"), str(tmp_path / "sampled")
+    code = ("import sys; sys.path.insert(0, %r); sys.path.insert(0, %r); from helpers import bench_emulation as be; "
+            "be.install(); import bench; be.run_own('config1_index_scatter', dump_outputs=%r); "
+            "bench.DUMP_BYTES = 1 << 20; be.run_own('config1_index_scatter', dump_outputs=%r)"
+            % (ROOT, os.path.join(ROOT, "tests"), whole, sampled))
+    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert sorted(os.listdir(whole)) == ["output.npy"] and sorted(os.listdir(sampled)) == ["output.npy", "output_rows.npy"]
+    full = np.load(os.path.join(whole, "output.npy"))
+    assert full.dtype == np.float32 and full.shape == (50_000, 64)        # config #1: S = 50,000 segments, F = 64
+    part, rows = np.load(os.path.join(sampled, "output.npy")), np.load(os.path.join(sampled, "output_rows.npy"))
+    assert part.dtype == np.float32 and rows.dtype == np.float64 and part.nbytes <= 1 << 20
+    assert part.shape == (rows.size, 64) and bool((np.diff(rows) > 0).all())
+    assert np.array_equal(part, full[rows.astype(np.int64)])
+    assert np.array_equal(full, _timed_output("config1_index_scatter")[1].numpy())
+
+
 @pytest.mark.parametrize("exchange", ["bucket", "allgather", "replicated"])
-def test_two_rank_flow_gloo(exchange):
+def test_two_rank_flow_gloo(exchange, tmp_path):
+    import numpy as np
     from helpers import bench_emulation as be
+    dump = str(tmp_path / "dump")
     s = socket.socket()
     s.bind(("127.0.0.1", 0))
     port = s.getsockname()[1]
     s.close()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
-    procs = [ctx.Process(target=be.worker, args=(r, 2, port, exchange, "arxiv_mh_spmm", q)) for r in range(2)]
+    procs = [ctx.Process(target=be.worker, args=(r, 2, port, exchange, "arxiv_mh_spmm", q, dump)) for r in range(2)]
     for p in procs:
         p.start()
     for p in procs:
@@ -62,3 +94,9 @@ def test_two_rank_flow_gloo(exchange):
     if exchange == "bucket":
         got, full = line["config"]["src_rows_received_per_step_rank0"], line["config"]["src_rows_full_exchange_rank0"]
         assert 0 < got == full
+    # --dump-outputs at N > 1: rank 0 writes the output assembled from both ranks' rows
+    part, rows = np.load(os.path.join(dump, "output.npy")), np.load(os.path.join(dump, "output_rows.npy")).astype(np.int64)
+    wk, exp = _timed_output("arxiv_mh_spmm")
+    assert part.dtype == np.float32 and part.shape == (rows.size, wk["H"], wk["F"]) and int(rows[-1]) < wk["S"]
+    exp = exp[torch.from_numpy(rows)].double()
+    assert bool(((torch.from_numpy(part).double() - exp).abs() <= 1e-2 * exp.abs().clamp_min(1e-3)).all())
