@@ -1,36 +1,26 @@
-// abi.cu -- the extern "C" boundary declared in include/geot_b200.h: argument checking, kernel shape
-// selection (replaces the reference's decision trees, csrc/cuda/wrapper/*_rule.h), format_preprocess
-// and the host-buffer entry.  No torch / ATen types here; the torch bindings (bindings.cpp) and any
-// other host (ctypes, cgo, JNI) call these functions.
+// abi.cu -- the extern "C" boundary declared in include/geot_b200.h for device buffers: argument checking, kernel
+// shape selection (replaces the reference's decision trees, csrc/cuda/wrapper/*_rule.h) and format_preprocess.  The
+// host-buffer entries are in host.cu.  No torch / ATen types here; the torch bindings (bindings.cpp) and any other
+// host (ctypes, cgo, JNI) call these functions.
 #include <cuda_runtime.h>
 #include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <algorithm>
-#include <thread>
-#include <vector>
 #include <cub/device/device_radix_sort.cuh>
 
-#include "../../include/geot_b200.h"
+#include "internal.h"
 #include "kernels/launch.h"
 
-namespace {
-
-thread_local char g_cuda_err[256] = "";
+static thread_local char g_cuda_err[256] = "";
 
 int cuda_fail(cudaError_t e, const char *what) {
   snprintf(g_cuda_err, sizeof(g_cuda_err), "%s: %s", what, cudaGetErrorString(e));
   return GEOT_ERR_CUDA;
 }
-#define CUDA_TRY(expr)                                    \
-  do {                                                    \
-    cudaError_t e__ = (expr);                             \
-    if (e__ != cudaSuccess) return cuda_fail(e__, #expr); \
-  } while (0)
 
-inline size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
-inline size_t dtype_size(int dt) { return dt == GEOT_F64 ? 8 : (dt == GEOT_F32 ? 4 : 2); }
+namespace {
+
 inline size_t acc_size(int dt) { return dt == GEOT_F64 ? 8 : 4; }
 inline int pow2ceil(int64_t x) { int p = 1; while (p < x) p <<= 1; return p; }
 
@@ -41,11 +31,6 @@ struct Config {
   int64_t tile_edges;
   int64_t n_tiles;
 };
-
-int env_int(const char *name, int dflt) {
-  const char *s = getenv(name);
-  return (s && *s) ? atoi(s) : dflt;
-}
 
 // `vector_ok`: rows are 16-byte addressable (per-head width multiple of the vector width and
 // 16-byte aligned base pointers); otherwise the element-wise kernels are used.
@@ -321,41 +306,6 @@ __global__ void csr_rows_kernel(const P *__restrict__ rowptr, int64_t S, int64_t
   row[e] = lo;
 }
 
-// fn(begin, end) over [0, n) on up to `threads` host threads (the calling thread takes the first share)
-template <typename F>
-void parallel_ranges(int threads, int64_t n, F fn) {
-  if (n <= 0) return;
-  threads = (int)std::max<int64_t>(1, std::min<int64_t>(threads, n / 4096 + 1));
-  if (threads == 1) { fn((int64_t)0, n); return; }
-  std::vector<std::thread> pool;
-  const int64_t per = (n + threads - 1) / threads;
-  for (int t = 1; t < threads; ++t) {
-    const int64_t b = per * t, e = std::min(n, b + per);
-    if (b < e) pool.emplace_back([=] { fn(b, e); });
-  }
-  fn((int64_t)0, std::min(n, per));
-  for (auto &th : pool) th.join();
-}
-
-// rp[i] = first position in idx[0, n) whose value is >= row0 + i, for i in [0, rows]  (idx sorted): the slice's CSR
-// row pointer.  Rows are walked in order, galloping from the previous boundary, so the cost follows the number of
-// cache lines a row spans rather than log2(n) misses per row.
-void host_row_pointers(const int64_t *idx, int64_t n, int64_t row0, int64_t rows, int64_t *rp, int threads) {
-  parallel_ranges(threads, rows + 1, [=](int64_t ia, int64_t ib) {
-    int64_t pos = std::lower_bound(idx, idx + n, row0 + ia) - idx;
-    for (int64_t i = ia; i < ib; ++i) {
-      const int64_t target = row0 + i;
-      if (pos < n && idx[pos] < target) {
-        int64_t lo = pos, step = 1;
-        while (lo + step < n && idx[lo + step] < target) { lo += step; step <<= 1; }
-        const int64_t hi = std::min(n, lo + step);
-        pos = std::lower_bound(idx + lo + 1, idx + hi, target) - idx;
-      }
-      rp[i] = pos;
-    }
-  });
-}
-
 // ---- instrumentation: event pairs around the main kernel ------------------------------------------
 struct Profile {
   int n = 0;
@@ -373,11 +323,6 @@ int bits_for(int64_t S) { int b = 1; while (b < 63 && ((int64_t)1 << b) < S) ++b
 
 // ==================================================================================================
 extern "C" {
-
-// used by the other translation units of the library (sddmm.cu); not exported
-__attribute__((visibility("hidden"))) int geot_b200_set_cuda_error(const char *what, int cuda_error) {
-  return cuda_fail((cudaError_t)cuda_error, what);
-}
 
 int geot_b200_version(void) { return GEOT_B200_VERSION; }
 int geot_b200_arch(void) { return 100; }
@@ -482,14 +427,6 @@ size_t geot_b200_workspace_bytes(int64_t E, int64_t W, int dtype, int sorted) {
 }
 
 }  // extern "C"
-
-namespace {
-// What the public entries do not expose: how empty rows are cleared and which rows the call owns.
-struct Extra {
-  int clear_mode = 0;          // 0: rows without edges are zeroed by this call; 1: the caller owns that (never clear)
-  int64_t fill_lo = 0;         // rows [fill_lo, fill_hi) belong to this call (host-entry slices); fill_hi < 0: [0, S)
-  int64_t fill_hi = -1;
-};
 
 int segment_reduce_impl(const void *src, const int64_t *src_index, const int64_t *dst_index,
                         const void *weight, void *dst, int64_t E, int64_t S, int64_t H, int64_t F,
@@ -652,7 +589,6 @@ int segment_reduce_impl(const void *src, const int64_t *src_index, const int64_t
   CUDA_TRY(launch(p, shape, stream, ev0, ev1));
   return GEOT_OK;
 }
-}  // namespace
 
 extern "C" {
 
@@ -772,401 +708,6 @@ int geot_b200_profile_read(float *ms, int capacity, int *count) {
     CUDA_TRY(cudaEventElapsedTime(&ms[i], g_prof.start[slot], g_prof.stop[slot]));
   }
   *count = k;
-  return GEOT_OK;
-}
-
-// ---- host-buffer entry ------------------------------------------------------------------------------
-// Pipeline: src first, then the sorted edge list in slices cut at segment boundaries.  Slice k+1 is
-// copied (H2D stream) while slice k is reduced (compute stream) and the finished dst rows of slice k-1
-// travel back (D2H stream, the other direction of the link).  Device buffers live in a per-process
-// arena that grows on demand and is reused across calls.
-namespace {
-struct Arena {
-  char *base = nullptr;
-  size_t bytes = 0;
-  cudaStream_t h2d = nullptr, comp = nullptr, d2h = nullptr;
-  static constexpr int kMaxSlices = 64;
-  cudaEvent_t copied[kMaxSlices] = {}, reduced[kMaxSlices] = {};
-  cudaEvent_t src_ready = nullptr;
-  char *pinned = nullptr;         // compact transport: host staging (row pointers, narrowed src ids), double-buffered
-  size_t pinned_bytes = 0;
-  unsigned long long last_h2d = 0, last_d2h = 0;   // bytes the last call moved over the link
-  int dev = -1;                   // the device the streams / buffers belong to
-};
-Arena g_arena;
-
-}  // namespace
-
-int geot_b200_host_arena_release(void) {
-  Arena &a = g_arena;
-  if (a.base) cudaFree(a.base);
-  if (a.pinned) cudaFreeHost(a.pinned);
-  for (int i = 0; i < Arena::kMaxSlices; ++i) {
-    if (a.copied[i]) cudaEventDestroy(a.copied[i]);
-    if (a.reduced[i]) cudaEventDestroy(a.reduced[i]);
-  }
-  if (a.src_ready) cudaEventDestroy(a.src_ready);
-  if (a.h2d) cudaStreamDestroy(a.h2d);
-  if (a.comp) cudaStreamDestroy(a.comp);
-  if (a.d2h) cudaStreamDestroy(a.d2h);
-  a = Arena();
-  return GEOT_OK;
-}
-
-int geot_b200_segment_reduce_host(const void *src, int64_t N_src, const int64_t *src_index,
-                                  const int64_t *dst_index, const void *weight, void *dst, int64_t E, int64_t S,
-                                  int64_t H, int64_t F, int dtype, int reduce, int weight_layout) {
-  if (!src || !dst_index || !dst || N_src <= 0) return GEOT_ERR_INVALID_ARG;
-  if (E <= 0) return GEOT_ERR_EMPTY;
-  if (S <= 0 || H <= 0 || F <= 0 || dtype < GEOT_F32 || dtype > GEOT_F16) return GEOT_ERR_INVALID_ARG;
-  if ((weight_layout == GEOT_W_NONE) != (weight == nullptr)) return GEOT_ERR_INVALID_ARG;
-  if (weight_layout == GEOT_W_HEAD_EDGE && H > 1) return GEOT_ERR_UNSUPPORTED;  // [H,E] cannot be sliced by edge
-  const int64_t W = H * F;
-  const size_t es = dtype_size(dtype);
-  const size_t wpe = weight ? (weight_layout == GEOT_W_EDGE ? 1 : (size_t)H) * es : 0;   // weight bytes per edge
-  const bool gather = src_index != nullptr;
-  const size_t b_src = (gather ? (size_t)N_src : 0) * W * es;   // index_scatter: src rows are edge-aligned, sliced
-  const size_t src_pe = gather ? 0 : (size_t)W * es;            // src bytes per edge when sliced
-  const size_t b_dst = (size_t)S * W * es;
-
-  // slices: about 128 MB of edge-aligned operands each, at least 4, cut at segment boundaries
-  const size_t per_edge = 8 + (gather ? 8 : 0) + wpe + src_pe;
-  int n_slices = (int)std::min<size_t>(Arena::kMaxSlices, std::max<size_t>(4, ((size_t)E * per_edge) >> 27));
-  if (E < 4096) n_slices = 1;
-  int64_t cut[Arena::kMaxSlices + 1];
-  cut[0] = 0;
-  int ns = 0;
-  for (int k = 1; k <= n_slices; ++k) {
-    int64_t c = (k == n_slices) ? E : (E / n_slices) * k;
-    while (c < E && c > 0 && dst_index[c] == dst_index[c - 1]) ++c;   // move right to a segment boundary
-    if (c > cut[ns]) cut[++ns] = c;
-    if (c >= E) break;
-  }
-  if (cut[ns] != E) cut[++ns] = E;
-  n_slices = ns;
-  int64_t max_slice = 0;
-  for (int k = 0; k < n_slices; ++k) max_slice = std::max(max_slice, cut[k + 1] - cut[k]);
-
-  // Row-pointer transport (default; GEOT_B200_HOST_COMPACT=0 turns it off): each slice sends its CSR row pointer
-  // (rows + 1 values, computed on the host threads while the previous slice is on the link) instead of its dst_index
-  // (one value per edge) and the device expands it.  Same results bit for bit; Reddit-shape gws moves 1.49 GB
-  // instead of 2.41 GB per call: 44.5 -> 28.1 ms (profiles/r02a_bench_compact*.json).  Narrowing src_index to int32
-  // on the host was measured too and lost (37.2 ms: the host pass costs more than the bytes it saves) -- removed.
-  const bool c_rows = env_int("GEOT_B200_HOST_COMPACT", 1) != 0;
-  int host_threads = env_int("GEOT_B200_HOST_THREADS", 0);
-  if (host_threads <= 0) host_threads = (int)std::min(32u, std::max(1u, std::thread::hardware_concurrency()));
-  int64_t max_rows = 0;   // rows of the widest slice: [first row of slice k (0 for k = 0), first row of slice k+1 (S at the end))
-  for (int k = 0; k < n_slices; ++k) {
-    const int64_t ra = (k == 0) ? 0 : dst_index[cut[k]], rb = (k + 1 < n_slices) ? dst_index[cut[k + 1]] : S;
-    max_rows = std::max(max_rows, rb - ra);
-  }
-  const size_t stage_rp = c_rows ? align256((size_t)(max_rows + 1) * 8) : 0;
-
-  // double-buffered slice operands + src + dst + workspace
-  const size_t slice_bytes = align256((size_t)max_slice * 8) * (gather ? 2 : 1) + align256((size_t)max_slice * wpe) +
-                             align256((size_t)max_slice * src_pe) + stage_rp;
-  const size_t b_ws = geot_b200_workspace_bytes(max_slice, W, dtype, 1);
-  const size_t total = align256(b_src) + align256(b_dst) + 2 * slice_bytes + align256(b_ws);
-  Arena &a = g_arena;
-  int rc = GEOT_OK;
-#define HOST_TRY(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) return cuda_fail(e__, #expr); } while (0)
-  int cur_dev = 0;
-  HOST_TRY(cudaGetDevice(&cur_dev));
-  if (a.dev >= 0 && a.dev != cur_dev) {      // the arena belongs to another device: start over on this one
-    int prev = a.dev;
-    cudaSetDevice(prev);
-    geot_b200_host_arena_release();
-    cudaSetDevice(cur_dev);
-  }
-  a.dev = cur_dev;
-  if (!a.h2d) {
-    HOST_TRY(cudaStreamCreateWithFlags(&a.h2d, cudaStreamNonBlocking));
-    HOST_TRY(cudaStreamCreateWithFlags(&a.comp, cudaStreamNonBlocking));
-    HOST_TRY(cudaStreamCreateWithFlags(&a.d2h, cudaStreamNonBlocking));
-    HOST_TRY(cudaEventCreateWithFlags(&a.src_ready, cudaEventDisableTiming));
-    for (int i = 0; i < Arena::kMaxSlices; ++i) {
-      HOST_TRY(cudaEventCreateWithFlags(&a.copied[i], cudaEventDisableTiming));
-      HOST_TRY(cudaEventCreateWithFlags(&a.reduced[i], cudaEventDisableTiming));
-    }
-  }
-  if (a.bytes < total) {
-    if (a.base) HOST_TRY(cudaFree(a.base));
-    a.base = nullptr; a.bytes = 0;
-    HOST_TRY(cudaMalloc(&a.base, total));
-    a.bytes = total;
-  }
-  if (a.pinned_bytes < 2 * stage_rp) {
-    if (a.pinned) HOST_TRY(cudaFreeHost(a.pinned));
-    a.pinned = nullptr; a.pinned_bytes = 0;
-    HOST_TRY(cudaHostAlloc(reinterpret_cast<void **>(&a.pinned), 2 * stage_rp, cudaHostAllocDefault));
-    a.pinned_bytes = 2 * stage_rp;
-  }
-  unsigned long long h2d_bytes = gather ? b_src : 0, d2h_bytes = 0;
-  char *p = a.base;
-  char *d_src = p; p += align256(b_src);
-  char *d_dst = p; p += align256(b_dst);
-  char *d_slice[2] = {p, p + slice_bytes}; p += 2 * slice_bytes;
-  void *d_ws = p;
-
-  HOST_TRY(cudaMemsetAsync(d_dst, 0, b_dst, a.comp));      // empty rows read 0; slices never clear
-  Extra never_clear;
-  never_clear.clear_mode = 1;
-  if (gather) HOST_TRY(cudaMemcpyAsync(d_src, src, b_src, cudaMemcpyHostToDevice, a.h2d));
-  HOST_TRY(cudaEventRecord(a.src_ready, a.h2d));
-  HOST_TRY(cudaStreamWaitEvent(a.comp, a.src_ready, 0));
-
-  for (int k = 0; k < n_slices; ++k) {
-    const int64_t e0 = cut[k], n = cut[k + 1] - cut[k];
-    char *q = d_slice[k & 1];
-    int64_t *s_di = reinterpret_cast<int64_t *>(q); q += align256((size_t)max_slice * 8);
-    int64_t *s_si = nullptr;
-    if (gather) { s_si = reinterpret_cast<int64_t *>(q); q += align256((size_t)max_slice * 8); }
-    char *s_w = q; q += align256((size_t)max_slice * wpe);
-    char *s_x = q; q += align256((size_t)max_slice * src_pe);
-    int64_t *s_rp = reinterpret_cast<int64_t *>(q);                         // row-pointer transport: device staging
-    // rows [first row of slice k, first row of slice k+1) belong to this slice
-    const int64_t r0 = dst_index[e0], r1 = (k + 1 < n_slices) ? dst_index[cut[k + 1]] : S;
-    const int64_t rr0 = (k == 0) ? 0 : r0;
-    // compact transport: the host threads prepare slice k while slice k-1 is on the link.  The pinned staging
-    // half is free once the copies of slice k-2 have left it.
-    char *hp = a.pinned + (size_t)(k & 1) * stage_rp;
-    int64_t *h_rp = reinterpret_cast<int64_t *>(hp);
-    if (c_rows && k >= 2) HOST_TRY(cudaEventSynchronize(a.copied[k - 2]));
-    if (c_rows) host_row_pointers(dst_index + e0, n, rr0, r1 - rr0, h_rp, host_threads);
-    // the buffer is free once slice k-2 has been reduced
-    if (k >= 2) HOST_TRY(cudaStreamWaitEvent(a.h2d, a.reduced[k - 2], 0));
-    if (c_rows) {
-      HOST_TRY(cudaMemcpyAsync(s_rp, h_rp, (size_t)(r1 - rr0 + 1) * 8, cudaMemcpyHostToDevice, a.h2d));
-      h2d_bytes += (size_t)(r1 - rr0 + 1) * 8;
-    } else {
-      HOST_TRY(cudaMemcpyAsync(s_di, dst_index + e0, (size_t)n * 8, cudaMemcpyHostToDevice, a.h2d));
-      h2d_bytes += (size_t)n * 8;
-    }
-    if (gather) {
-      HOST_TRY(cudaMemcpyAsync(s_si, src_index + e0, (size_t)n * 8, cudaMemcpyHostToDevice, a.h2d));
-      h2d_bytes += (size_t)n * 8;
-    }
-    if (weight) HOST_TRY(cudaMemcpyAsync(s_w, static_cast<const char *>(weight) + (size_t)e0 * wpe, (size_t)n * wpe, cudaMemcpyHostToDevice, a.h2d));
-    if (!gather) HOST_TRY(cudaMemcpyAsync(s_x, static_cast<const char *>(src) + (size_t)e0 * src_pe, (size_t)n * src_pe, cudaMemcpyHostToDevice, a.h2d));
-    h2d_bytes += (size_t)n * (wpe + src_pe);
-    HOST_TRY(cudaEventRecord(a.copied[k], a.h2d));
-    HOST_TRY(cudaStreamWaitEvent(a.comp, a.copied[k], 0));
-    const unsigned nb = (unsigned)((n + 255) / 256);
-    if (c_rows) {   // expand the row pointer into slice-local dst ids [0, r1 - rr0)
-      csr_rows_kernel<int64_t><<<nb, 256, 0, a.comp>>>(s_rp, r1 - rr0, n, s_di);
-      HOST_TRY(cudaGetLastError());
-    }
-    if (c_rows)     // slice-local dst ids: the slice's rows start at d_dst + rr0 * W
-      rc = segment_reduce_impl(gather ? d_src : s_x, s_si, s_di, weight ? s_w : nullptr, d_dst + (size_t)rr0 * W * es, n, r1 - rr0,
-                               H, F, dtype, reduce, weight_layout, 1, nullptr, d_ws, b_ws, a.comp, nullptr, never_clear);
-    else
-      rc = segment_reduce_impl(gather ? d_src : s_x, s_si, s_di, weight ? s_w : nullptr, d_dst, n, S, H, F, dtype, reduce,
-                               weight_layout, 1, nullptr, d_ws, b_ws, a.comp, nullptr, never_clear);
-    if (rc != GEOT_OK) { cudaDeviceSynchronize(); return rc; }
-    HOST_TRY(cudaEventRecord(a.reduced[k], a.comp));
-    // rows [rr0, r1) are final: send them home
-    HOST_TRY(cudaStreamWaitEvent(a.d2h, a.reduced[k], 0));
-    d2h_bytes += (size_t)(r1 - rr0) * W * es;
-    HOST_TRY(cudaMemcpyAsync(static_cast<char *>(dst) + (size_t)rr0 * W * es, d_dst + (size_t)rr0 * W * es,
-                             (size_t)(r1 - rr0) * W * es, cudaMemcpyDeviceToHost, a.d2h));
-  }
-  HOST_TRY(cudaStreamSynchronize(a.d2h));
-  HOST_TRY(cudaStreamSynchronize(a.comp));
-  HOST_TRY(cudaStreamSynchronize(a.h2d));
-#undef HOST_TRY
-  a.last_h2d = h2d_bytes;
-  a.last_d2h = d2h_bytes;
-  return rc;
-}
-
-// ---- resident host graph -------------------------------------------------------------------------------
-// The graph (index arrays) of a GNN is static across layers and epochs while the features and edge weights change
-// every call.  A host graph handle uploads the indices ONCE; every reduce call then ships only src (+ weights) over
-// the link and brings dst back: Reddit-shape gather_weight_scatter moves 0.58 GB per call instead of 2.41 GB.
-struct geot_host_graph {
-  int dev = 0;
-  int64_t E = 0, S = 0, N_src = 0;
-  bool gather = false;
-  int64_t *d_di = nullptr, *d_si = nullptr;     // resident indices
-  static constexpr int kFine = 256;             // fine cuts at segment boundaries; a call groups them into slices
-  int n_fine = 0;
-  int64_t cut[kFine + 1];                       // edge offsets
-  int64_t row_cut[kFine + 1];                   // first dst row of every fine slice (row_cut[0] = 0, row_cut[n_fine] = S)
-  char *work = nullptr;                         // per-call device buffers, grown on demand
-  size_t work_bytes = 0;
-  cudaStream_t h2d = nullptr, comp = nullptr, d2h = nullptr;
-  static constexpr int kMaxSlices = 64;
-  cudaEvent_t copied[kMaxSlices] = {}, reduced[kMaxSlices] = {};
-  cudaEvent_t src_ready = nullptr;
-  unsigned long long last_h2d = 0, last_d2h = 0, resident_bytes = 0;
-};
-
-int geot_b200_host_graph_destroy(geot_host_graph_t *g) {
-  if (!g) return GEOT_OK;
-  int cur = 0;
-  cudaGetDevice(&cur);
-  cudaSetDevice(g->dev);
-  if (g->d_di) cudaFree(g->d_di);
-  if (g->d_si) cudaFree(g->d_si);
-  if (g->work) cudaFree(g->work);
-  for (int i = 0; i < geot_host_graph::kMaxSlices; ++i) {
-    if (g->copied[i]) cudaEventDestroy(g->copied[i]);
-    if (g->reduced[i]) cudaEventDestroy(g->reduced[i]);
-  }
-  if (g->src_ready) cudaEventDestroy(g->src_ready);
-  if (g->h2d) cudaStreamDestroy(g->h2d);
-  if (g->comp) cudaStreamDestroy(g->comp);
-  if (g->d2h) cudaStreamDestroy(g->d2h);
-  cudaSetDevice(cur);
-  delete g;
-  return GEOT_OK;
-}
-
-int geot_b200_host_graph_create(const int64_t *src_index, const int64_t *dst_index, int64_t E, int64_t S, int64_t N_src,
-                                geot_host_graph_t **out) {
-  if (!dst_index || !out || S <= 0 || (src_index && N_src <= 0)) return GEOT_ERR_INVALID_ARG;
-  if (E <= 0) return GEOT_ERR_EMPTY;
-  if (dst_index[E - 1] >= S || dst_index[0] < 0) return GEOT_ERR_INVALID_ARG;
-  geot_host_graph *g = new geot_host_graph();
-#define G_TRY(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) { int rc__ = cuda_fail(e__, #expr); geot_b200_host_graph_destroy(g); return rc__; } } while (0)
-  G_TRY(cudaGetDevice(&g->dev));
-  g->E = E; g->S = S; g->N_src = N_src; g->gather = src_index != nullptr;
-  G_TRY(cudaStreamCreateWithFlags(&g->h2d, cudaStreamNonBlocking));
-  G_TRY(cudaStreamCreateWithFlags(&g->comp, cudaStreamNonBlocking));
-  G_TRY(cudaStreamCreateWithFlags(&g->d2h, cudaStreamNonBlocking));
-  G_TRY(cudaEventCreateWithFlags(&g->src_ready, cudaEventDisableTiming));
-  for (int i = 0; i < geot_host_graph::kMaxSlices; ++i) {
-    G_TRY(cudaEventCreateWithFlags(&g->copied[i], cudaEventDisableTiming));
-    G_TRY(cudaEventCreateWithFlags(&g->reduced[i], cudaEventDisableTiming));
-  }
-  G_TRY(cudaMalloc(&g->d_di, (size_t)E * 8));
-  G_TRY(cudaMemcpyAsync(g->d_di, dst_index, (size_t)E * 8, cudaMemcpyHostToDevice, g->h2d));
-  g->resident_bytes = (size_t)E * 8;
-  if (src_index) {
-    G_TRY(cudaMalloc(&g->d_si, (size_t)E * 8));
-    G_TRY(cudaMemcpyAsync(g->d_si, src_index, (size_t)E * 8, cudaMemcpyHostToDevice, g->h2d));
-    g->resident_bytes += (size_t)E * 8;
-  }
-  // fine cuts: about E / kFine edges each, moved right to a segment boundary (while the copies run)
-  const int want = (int)std::min<int64_t>(geot_host_graph::kFine, std::max<int64_t>(1, E / 65536));
-  g->cut[0] = 0;
-  g->row_cut[0] = 0;
-  int ns = 0;
-  for (int k = 1; k <= want; ++k) {
-    int64_t c = (k == want) ? E : (E / want) * k;
-    while (c < E && c > 0 && dst_index[c] == dst_index[c - 1]) ++c;
-    if (c > g->cut[ns]) {
-      ++ns;
-      g->cut[ns] = c;
-      g->row_cut[ns] = (c < E) ? dst_index[c] : S;
-    }
-    if (c >= E) break;
-  }
-  g->n_fine = ns;
-  G_TRY(cudaStreamSynchronize(g->h2d));
-#undef G_TRY
-  *out = g;
-  return GEOT_OK;
-}
-
-int geot_b200_host_graph_reduce(geot_host_graph_t *g, const void *src, const void *weight, void *dst, int64_t H,
-                                int64_t F, int dtype, int reduce, int weight_layout) {
-  if (!g || !src || !dst) return GEOT_ERR_INVALID_ARG;
-  if (H <= 0 || F <= 0 || dtype < GEOT_F32 || dtype > GEOT_F16) return GEOT_ERR_INVALID_ARG;
-  if ((weight_layout == GEOT_W_NONE) != (weight == nullptr)) return GEOT_ERR_INVALID_ARG;
-  if (weight_layout == GEOT_W_HEAD_EDGE && H > 1) return GEOT_ERR_UNSUPPORTED;  // [H,E] cannot be sliced by edge
-  int cur_dev = 0;
-#define HOST_TRY(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) return cuda_fail(e__, #expr); } while (0)
-  HOST_TRY(cudaGetDevice(&cur_dev));
-  if (cur_dev != g->dev) return GEOT_ERR_INVALID_ARG;       // the handle lives on the device it was created on
-  const int64_t E = g->E, S = g->S, W = H * F;
-  const size_t es = dtype_size(dtype);
-  const size_t wpe = weight ? (weight_layout == GEOT_W_EDGE ? 1 : (size_t)H) * es : 0;
-  const size_t src_pe = g->gather ? 0 : (size_t)W * es;
-  const size_t b_src = g->gather ? (size_t)g->N_src * W * es : 0;
-  const size_t b_dst = (size_t)S * W * es;
-
-  // group the fine cuts into slices of about 48 MB of per-edge payload (at least 4 when the graph allows, at most 64)
-  const size_t per_edge = std::max<size_t>(wpe + src_pe, 1);
-  int n_slices = (int)std::min<size_t>(geot_host_graph::kMaxSlices, std::max<size_t>(4, ((size_t)E * per_edge) / (48u << 20)));
-  n_slices = std::min(n_slices, g->n_fine);
-  int first[geot_host_graph::kMaxSlices + 1];
-  for (int k = 0; k <= n_slices; ++k) first[k] = (int)(((int64_t)g->n_fine * k) / n_slices);
-  int64_t max_slice = 0;
-  for (int k = 0; k < n_slices; ++k) max_slice = std::max(max_slice, g->cut[first[k + 1]] - g->cut[first[k]]);
-
-  const size_t slice_bytes = align256((size_t)max_slice * wpe) + align256((size_t)max_slice * src_pe);
-  const size_t b_ws = geot_b200_workspace_bytes(max_slice, W, dtype, 1);
-  const size_t total = align256(b_src) + align256(b_dst) + 2 * slice_bytes + align256(b_ws);
-  if (g->work_bytes < total) {
-    if (g->work) HOST_TRY(cudaFree(g->work));
-    g->work = nullptr; g->work_bytes = 0;
-    HOST_TRY(cudaMalloc(&g->work, total));
-    g->work_bytes = total;
-  }
-  char *p = g->work;
-  char *d_src = p; p += align256(b_src);
-  char *d_dst = p; p += align256(b_dst);
-  char *d_slice[2] = {p, p + slice_bytes}; p += 2 * slice_bytes;
-  void *d_ws = p;
-  unsigned long long h2d_bytes = b_src, d2h_bytes = 0;
-
-  if (g->gather) HOST_TRY(cudaMemcpyAsync(d_src, src, b_src, cudaMemcpyHostToDevice, g->h2d));
-  HOST_TRY(cudaEventRecord(g->src_ready, g->h2d));
-  HOST_TRY(cudaStreamWaitEvent(g->comp, g->src_ready, 0));
-  int rc = GEOT_OK;
-  for (int k = 0; k < n_slices; ++k) {
-    const int64_t e0 = g->cut[first[k]], n = g->cut[first[k + 1]] - e0;
-    const int64_t r0 = g->row_cut[first[k]], r1 = g->row_cut[first[k + 1]];     // this slice owns rows [r0, r1)
-    char *q = d_slice[k & 1];
-    char *s_w = q; q += align256((size_t)max_slice * wpe);
-    char *s_x = q;
-    if (k >= 2) HOST_TRY(cudaStreamWaitEvent(g->h2d, g->reduced[k - 2], 0));   // the buffer half is free again
-    if (weight) HOST_TRY(cudaMemcpyAsync(s_w, static_cast<const char *>(weight) + (size_t)e0 * wpe, (size_t)n * wpe, cudaMemcpyHostToDevice, g->h2d));
-    if (!g->gather) HOST_TRY(cudaMemcpyAsync(s_x, static_cast<const char *>(src) + (size_t)e0 * src_pe, (size_t)n * src_pe, cudaMemcpyHostToDevice, g->h2d));
-    h2d_bytes += (size_t)n * (wpe + src_pe);
-    HOST_TRY(cudaEventRecord(g->copied[k], g->h2d));
-    HOST_TRY(cudaStreamWaitEvent(g->comp, g->copied[k], 0));
-    Extra ex;                      // rows without edges inside [r0, r1) are zero-filled by the kernel: no memset
-    ex.fill_lo = r0;
-    ex.fill_hi = r1;
-    rc = segment_reduce_impl(g->gather ? d_src : s_x, g->gather ? g->d_si + e0 : nullptr, g->d_di + e0, weight ? s_w : nullptr,
-                             d_dst, n, S, H, F, dtype, reduce, weight_layout, 1, nullptr, d_ws, b_ws, g->comp, nullptr, ex);
-    if (rc != GEOT_OK) { cudaDeviceSynchronize(); return rc; }
-    HOST_TRY(cudaEventRecord(g->reduced[k], g->comp));
-    HOST_TRY(cudaStreamWaitEvent(g->d2h, g->reduced[k], 0));
-    d2h_bytes += (size_t)(r1 - r0) * W * es;
-    HOST_TRY(cudaMemcpyAsync(static_cast<char *>(dst) + (size_t)r0 * W * es, d_dst + (size_t)r0 * W * es,
-                             (size_t)(r1 - r0) * W * es, cudaMemcpyDeviceToHost, g->d2h));
-  }
-  HOST_TRY(cudaStreamSynchronize(g->d2h));
-  HOST_TRY(cudaStreamSynchronize(g->comp));
-  HOST_TRY(cudaStreamSynchronize(g->h2d));
-#undef HOST_TRY
-  g->last_h2d = h2d_bytes;
-  g->last_d2h = d2h_bytes;
-  return rc;
-}
-
-int geot_b200_host_graph_last_transfer(const geot_host_graph_t *g, unsigned long long *h2d_bytes, unsigned long long *d2h_bytes,
-                                       unsigned long long *resident_bytes) {
-  if (!g) return GEOT_ERR_INVALID_ARG;
-  if (h2d_bytes) *h2d_bytes = g->last_h2d;
-  if (d2h_bytes) *d2h_bytes = g->last_d2h;
-  if (resident_bytes) *resident_bytes = g->resident_bytes;
-  return GEOT_OK;
-}
-
-int geot_b200_host_row_pointers(const int64_t *index, int64_t n, int64_t row0, int64_t rows, int64_t *rowptr, int threads) {
-  if (!index || !rowptr || n < 0 || rows < 0) return GEOT_ERR_INVALID_ARG;
-  if (threads <= 0) threads = (int)std::min(32u, std::max(1u, std::thread::hardware_concurrency()));
-  host_row_pointers(index, n, row0, rows, rowptr, threads);
-  return GEOT_OK;
-}
-
-int geot_b200_host_last_transfer(unsigned long long *h2d_bytes, unsigned long long *d2h_bytes) {
-  if (h2d_bytes) *h2d_bytes = g_arena.last_h2d;
-  if (d2h_bytes) *d2h_bytes = g_arena.last_d2h;
   return GEOT_OK;
 }
 

@@ -14,13 +14,9 @@
 
 #include <cub/device/device_radix_sort.cuh>
 
-#include "../../include/geot_b200.h"
-
-extern "C" int geot_b200_set_cuda_error(const char *what, int cuda_error);
+#include "internal.h"
 
 namespace {
-
-inline size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
 
 // key[e] = block of src_index[e]; val[e] = e; per-block edge counts
 __global__ void __launch_bounds__(256)
@@ -102,7 +98,6 @@ int geot_b200_src_blocks_build(const int64_t *src_index, const int64_t *dst_inde
   if (buf_bytes < geot_b200_src_blocks_bytes(E) || scratch_bytes < geot_b200_src_blocks_scratch_bytes(E) ||
       ((reinterpret_cast<uintptr_t>(buf) | reinterpret_cast<uintptr_t>(scratch)) & 255))
     return GEOT_ERR_WORKSPACE;
-#define B_TRY(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) return geot_b200_set_cuda_error(#expr, (int)e__); } while (0)
   char *p = static_cast<char *>(buf);
   int64_t *dst_b = reinterpret_cast<int64_t *>(p); p += align256((size_t)E * 8);
   int64_t *src_b = reinterpret_cast<int64_t *>(p); p += align256((size_t)E * 8);
@@ -115,20 +110,19 @@ int geot_b200_src_blocks_build(const int64_t *src_index, const int64_t *dst_inde
   void *cub_tmp = q;
   size_t cb = cub_bytes(E);
   const int64_t rows_per_block = (N_src + n_blocks - 1) / n_blocks;
-  B_TRY(cudaMemsetAsync(counts, 0, GEOT_MAX_SRC_BLOCKS * 8, stream));
+  CUDA_TRY(cudaMemsetAsync(counts, 0, GEOT_MAX_SRC_BLOCKS * 8, stream));
   const unsigned nb = (unsigned)std::min<int64_t>((E + 255) / 256, 148 * 16);
   block_keys_kernel<<<nb, 256, 0, stream>>>(src_index, E, rows_per_block, n_blocks, key_in, val_in, counts);
-  B_TRY(cudaGetLastError());
+  CUDA_TRY(cudaGetLastError());
   int bits = 1;
   while ((1 << bits) < n_blocks) ++bits;
   // LSD radix sort on the block id: stable, so every block keeps the (dst, src) order of the caller's list
-  B_TRY(cub::DeviceRadixSort::SortPairs(cub_tmp, cb, key_in, key_out, val_in, perm, E, 0, bits, stream));
+  CUDA_TRY(cub::DeviceRadixSort::SortPairs(cub_tmp, cb, key_in, key_out, val_in, perm, E, 0, bits, stream));
   regroup_kernel<<<nb, 256, 0, stream>>>(perm, src_index, dst_index, E, src_b, dst_b);
-  B_TRY(cudaGetLastError());
+  CUDA_TRY(cudaGetLastError());
   unsigned long long h[GEOT_MAX_SRC_BLOCKS];
-  B_TRY(cudaMemcpyAsync(h, counts, sizeof(h), cudaMemcpyDeviceToHost, stream));
-  B_TRY(cudaStreamSynchronize(stream));
-#undef B_TRY
+  CUDA_TRY(cudaMemcpyAsync(h, counts, sizeof(h), cudaMemcpyDeviceToHost, stream));
+  CUDA_TRY(cudaStreamSynchronize(stream));
   out->E = E;
   out->n_blocks = n_blocks;
   out->reserved = 0;

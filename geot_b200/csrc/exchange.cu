@@ -12,9 +12,7 @@
 #include <stdint.h>
 #include <stdlib.h>
 
-#include "../../include/geot_b200.h"
-
-extern "C" int geot_b200_set_cuda_error(const char *what, int cuda_error);
+#include "internal.h"
 
 namespace {
 
@@ -118,7 +116,7 @@ int geot_b200_permute_edges(const void *in, const int64_t *perm, void *out, int6
     permute_edges16_kernel<<<blocks, 256, 0, stream>>>(static_cast<const uint16_t *>(in), perm, static_cast<uint16_t *>(out),
                                                        E, (int)(bytes_per_edge / 2));
   cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return geot_b200_set_cuda_error("permute_edges_kernel", (int)e);
+  if (e != cudaSuccess) return cuda_fail(e, "permute_edges_kernel");
   return GEOT_OK;
 }
 
@@ -159,7 +157,7 @@ int geot_b200_push_rows_ex(const void *x, const int64_t *rows, const int32_t *de
                                                                     reinterpret_cast<uint16_t *const *>(peer_bases), n, (int)vecs,
                                                                     shift);
   cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return geot_b200_set_cuda_error("push_rows_kernel", (int)e);
+  if (e != cudaSuccess) return cuda_fail(e, "push_rows_kernel");
   return GEOT_OK;
 }
 

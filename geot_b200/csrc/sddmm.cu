@@ -3,7 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdio.h>
 
-#include "../../include/geot_b200.h"
+#include "internal.h"
 #include "kernels/sddmm.cuh"
 
 namespace geot {
@@ -69,8 +69,6 @@ cudaError_t launch_sddmm_type(const SddmmParams &p, bool vector_ok, cudaStream_t
 }  // namespace
 }  // namespace geot
 
-extern "C" int geot_b200_set_cuda_error(const char *what, int cuda_error);   // abi.cu
-
 extern "C" int geot_b200_sddmm_coo(const void *mat1, const int64_t *row_index, const void *mat2, const int64_t *col_index,
                                    void *out, int64_t E, int64_t F, int dtype, cudaStream_t stream) {
   if (E < 0 || F <= 0 || dtype < GEOT_F32 || dtype > GEOT_F16) return GEOT_ERR_INVALID_ARG;
@@ -87,6 +85,6 @@ extern "C" int geot_b200_sddmm_coo(const void *mat1, const int64_t *row_index, c
     case GEOT_BF16: e = geot::launch_sddmm_type<__nv_bfloat16>(p, aligned, stream); break;
     default: e = geot::launch_sddmm_type<__half>(p, aligned, stream); break;
   }
-  if (e != cudaSuccess) return geot_b200_set_cuda_error("sddmm_coo launch", (int)e);
+  if (e != cudaSuccess) return cuda_fail(e, "sddmm_coo launch");
   return GEOT_OK;
 }

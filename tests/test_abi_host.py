@@ -73,6 +73,21 @@ def test_argument_validation_happens_before_any_device_work():
     assert f(one, null, one, null, one, 10, 4, 1, 8, abi.F32, abi.SUM, abi.W_NONE, 1, None, ctypes.c_void_p(264), 1 << 20, null) == 3  # misaligned ws
     assert L.geot_b200_gather_scatter(one, null, one, one, 10, 4, 8, abi.F32, abi.SUM, None, one, 1 << 20, null) == 1  # src_index missing
     assert L.geot_b200_mh_spmm(one, one, one, one, one, 10, 4, 2, 8, abi.F32, abi.SUM, abi.W_EDGE, None, one, 1 << 20, null) == 1
+    # host-buffer entries: the row ranges of the slices come from dst_index read at 0, at every cut and at E-1, so an
+    # index that leaves [0, S) or decreases there is refused before any CUDA call
+    E = 8192
+    di = torch.arange(E) // 4
+    S = int(di[-1]) + 1
+    neg = di.clone()
+    neg[0] = -1
+    rotated = di.roll(E // 2)
+    host = L.geot_b200_segment_reduce_host
+    for idx, rows in ((di, S - 1), (neg, S), (rotated, S)):
+        assert host(one, S, one, idx.data_ptr(), null, one, E, rows, 1, 8, abi.F32, abi.SUM, abi.W_NONE) == 1
+    big = (torch.arange(200_000) // 4).roll(100_000)
+    h = ctypes.c_void_p(0)
+    assert L.geot_b200_host_graph_create(one, big.data_ptr(), big.numel(), 50_000, 50_000, ctypes.byref(h)) == 1
+    assert not h.value
     with pytest.raises(abi.AbiError, match="invalid argument"):
         abi.check(1, "x")
 
