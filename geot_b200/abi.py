@@ -22,7 +22,7 @@ SYMBOLS = [
     "geot_b200_index_last", "geot_b200_plan_bytes", "geot_b200_format_preprocess", "geot_b200_plan_shards",
     "geot_b200_workspace_bytes", "geot_b200_segment_reduce", "geot_b200_index_scatter",
     "geot_b200_gather_scatter", "geot_b200_gather_weight_scatter", "geot_b200_mh_spmm",
-    "geot_b200_sddmm_coo", "geot_b200_csr_to_coo", "geot_b200_permute_edges",
+    "geot_b200_sddmm_coo", "geot_b200_sddmm_mh", "geot_b200_csr_to_coo", "geot_b200_permute_edges",
     "geot_b200_segment_reduce_host", "geot_b200_host_arena_release", "geot_b200_profile_enable", "geot_b200_profile_read",
     "geot_b200_push_rows", "geot_b200_push_rows_ex", "geot_b200_set_unsorted_mode",
     "geot_b200_host_last_transfer", "geot_b200_host_row_pointers", "geot_b200_segment_reduce_ex",
@@ -99,6 +99,7 @@ def lib() -> ctypes.CDLL:
         L.geot_b200_mh_spmm.argtypes = [vp, vp, vp, vp, vp, i64, i64, i64, i64, ci, ci, ci,
                                         ctypes.POINTER(GeotPlan), vp, sz, vp]
         L.geot_b200_sddmm_coo.argtypes = [vp, vp, vp, vp, vp, i64, i64, ci, vp]
+        L.geot_b200_sddmm_mh.argtypes = [vp, vp, vp, vp, vp, i64, i64, i64, ci, ci, vp]
         L.geot_b200_csr_to_coo.argtypes = [vp, ci, i64, i64, vp, vp]
         L.geot_b200_permute_edges.argtypes = [vp, vp, vp, i64, i64, vp]
         L.geot_b200_segment_reduce_host.argtypes = [vp, i64, vp, vp, vp, vp, i64, i64, i64, i64, ci, ci, ci]
@@ -242,6 +243,16 @@ def sddmm_coo(mat1, row_index, mat2, col_index):
     out = torch.empty(E, dtype=mat1.dtype, device=mat1.device)
     check(lib().geot_b200_sddmm_coo(_ptr(mat1), _ptr(row_index), _ptr(mat2), _ptr(col_index), _ptr(out), E,
                                     mat1.shape[1], DTYPE[mat1.dtype], _stream()), "sddmm_coo")
+    return out
+
+
+def sddmm_mh(mat1, row_index, mat2, col_index, head_major=False):
+    """out[e, h] = <mat1[row_index[e], h], mat2[col_index[e], h]> ([E, H], or [H, E] with head_major) through
+    geot_b200_sddmm_mh; mat1 / mat2 [N, H, F]."""
+    E, H, F = row_index.numel(), mat1.shape[1], mat1.shape[2]
+    out = torch.empty([H, E] if head_major else [E, H], dtype=mat1.dtype, device=mat1.device)
+    check(lib().geot_b200_sddmm_mh(_ptr(mat1), _ptr(row_index), _ptr(mat2), _ptr(col_index), _ptr(out), E, H, F,
+                                   DTYPE[mat1.dtype], W_HEAD_EDGE if head_major else W_EDGE_HEAD, _stream()), "sddmm_mh")
     return out
 
 

@@ -397,6 +397,29 @@ at::Tensor sddmm_coo_impl(at::Tensor src_index, at::Tensor dst_index, at::Tensor
   return out;
 }
 
+// geot::sddmm_mh_impl -- the weight gradient of mh_spmm: out[e, h] = <mat_1[dst_index[e], h, :], mat_2[src_index[e], h, :]>,
+// [E, H], or [H, E] with head_major (the two weight layouts of mh_spmm).  Checks as sddmm_coo_impl.
+at::Tensor sddmm_mh_impl(at::Tensor src_index, at::Tensor dst_index, at::Tensor mat_1, at::Tensor mat_2, bool head_major) {
+  TORCH_CHECK(mat_1.is_cuda() && mat_2.is_cuda(), "geot::sddmm_mh: mat_1 and mat_2 must be CUDA tensors (this build has no CPU path)");
+  TORCH_CHECK(src_index.dim() == 1 && dst_index.dim() == 1 && src_index.numel() == dst_index.numel(),
+              "src_index and dst_index must be 1 dimensional and of the same length");
+  TORCH_CHECK(mat_1.dim() == 3 && mat_2.dim() == 3 && mat_1.size(1) == mat_2.size(1) && mat_1.size(2) == mat_2.size(2),
+              "mat_1 and mat_2 must be 3 dimensional [N, H, F] with the same H and F");
+  TORCH_CHECK(mat_1.scalar_type() == mat_2.scalar_type(), "mat_1 and mat_2 must have the same dtype");
+  c10::cuda::CUDAGuard guard(mat_1.device());
+  const at::Tensor col = src_index.to(at::kLong).contiguous(), row = dst_index.to(at::kLong).contiguous();
+  TORCH_CHECK(row.is_cuda() && col.is_cuda(), "geot::sddmm_mh: indices must be CUDA tensors");
+  const at::Tensor a = mat_1.contiguous(), b = mat_2.contiguous();
+  const int64_t E = row.numel(), H = a.size(1), F = a.size(2);
+  TORCH_CHECK(H > 0 && F > 0, "geot::sddmm_mh: mat_1 and mat_2 must have at least one head and one feature");
+  at::Tensor out = head_major ? at::empty({H, E}, a.options()) : at::empty({E, H}, a.options());
+  check_status(geot_b200_sddmm_mh(a.data_ptr(), row.data_ptr<int64_t>(), b.data_ptr(), col.data_ptr<int64_t>(), out.data_ptr(), E,
+                                  H, F, dtype_enum(a), head_major ? GEOT_W_HEAD_EDGE : GEOT_W_EDGE_HEAD,
+                                  at::cuda::getCurrentCUDAStream()),
+               "sddmm_mh");
+  return out;
+}
+
 // ---- CSR entry point ------------------------------------------------------------------------------------
 // Cache of the COO row index expanded from a CSR row pointer, keyed like the plans (storage + version).
 struct CsrEntry {
@@ -497,6 +520,7 @@ TORCH_LIBRARY_FRAGMENT(geot, m) {
   m.def("gather_weight_scatter_reduce(Tensor src_index, Tensor dst_index, Tensor weight, Tensor src, str reduce) -> Tensor");
   m.def("format_preprocess(Tensor dst_index) -> (Tensor, Tensor)");
   m.def("plan_shards(Tensor dst_index, int parts) -> Tensor");
+  m.def("sddmm_mh_impl(Tensor src_index, Tensor dst_index, Tensor mat_1, Tensor mat_2, bool head_major) -> Tensor");
   m.def("clear_plan_cache() -> ()", []() { clear_plan_cache(); });
   m.def("abi_version() -> int", []() { return (int64_t)geot_b200_version(); });
 }
@@ -513,4 +537,5 @@ TORCH_LIBRARY_IMPL(geot, CUDA, m) {
   m.impl("gather_weight_scatter_reduce", gather_weight_scatter_reduce);
   m.impl("format_preprocess", format_preprocess);
   m.impl("plan_shards", plan_shards);
+  m.impl("sddmm_mh_impl", sddmm_mh_impl);
 }

@@ -1,7 +1,8 @@
-// sddmm.cuh -- sampled dense-dense product on a COO edge list, sm_100a:
+// sddmm.cuh -- sampled dense-dense product on a COO edge list, sm_100a, one dot product per edge and head:
 //
-//     out[e] = < mat1[row_index[e], :] , mat2[col_index[e], :] >          e = 0 .. E-1
+//     out[e, h] = < mat1[row_index[e], h, :] , mat2[col_index[e], h, :] >   e = 0 .. E-1,  h = 0 .. H-1
 //
+// H = 1 is the weight gradient of gather_weight_scatter; H > 1 (rows of W = H*F elements) that of mh_spmm.
 // Replaces the reference's sddmm_coo_ebalance_{vec4,vec2,scalar} (csrc/cuda/sddmm_coo_kernel.cuh:3-215,
 // launcher csrc/cuda/gather_weight_scatter_cuda.cu:41-62), which serve the weight gradient of
 // gather_weight_scatter (geot/gather_weight_scatter.py:47).  The reference is fp32 + int32 only and
@@ -19,7 +20,11 @@
 //     unaligned data -- double-buffered in registers;
 //   * the U per-lane partial dot products are reduced across the group with a transposing butterfly
 //     (U - 1 + log2(LPR/U) shuffles per U edges instead of U * log2(LPR)), after which lane k*(LPR/U)
-//     holds edge k's result: U consecutive outputs = one 32-byte sector.
+//     holds edge k's result: U consecutive outputs = one 32-byte sector;
+//   * H > 1: a head is HV whole vectors (HV a power of two).  With HV <= LPR the butterfly runs over the low log2(HV)
+//     lane bits only and a lane keeps one partial per vector it holds (each of its VPL vectors is in another head);
+//     the results are then gathered so that the LPR * H outputs of a batch leave in coalesced stores, as [E,H] (the
+//     H results of an edge contiguous) or [H,E] (the edges of a head contiguous).
 #pragma once
 #include "segment_reduce.cuh"
 
@@ -30,17 +35,19 @@ struct SddmmParams {
   const void *mat2;             // [N2, W], indexed by col_index
   const int64_t *row_index;     // [E]
   const int64_t *col_index;     // [E]
-  void *out;                    // [E]
+  void *out;                    // [E, H], or [H, E] with head_major
   int64_t E;
-  int64_t W;
+  int64_t W;                    // H * F
+  int64_t H;
+  int head_major;
   int chunk_edges;
 };
 
-// Transposing butterfly over a group of LPR lanes: p[0..U) per lane in, and on return p[0] of lane gl
-// holds the group-wide sum of value (gl / (LPR / U)).
+// Transposing butterfly over the low log2(LPR) lane bits: p[0..U) per lane in.  On return, with U <= LPR, p[0] of lane
+// gl holds the sum over its LPR lanes of value ((gl % LPR) / (LPR / U)); with U > LPR, p[0 .. U/LPR) hold values
+// (gl % LPR) * (U / LPR) + 0 .. U/LPR-1.
 template <int U, int LPR, typename A>
 __device__ __forceinline__ void group_transpose_reduce(A (&p)[U], unsigned gmask, int gl) {
-  static_assert(U <= LPR, "U values need at least U lanes");
   int n = U;
 #pragma unroll
   for (int s = LPR / 2; s >= 1; s >>= 1) {
@@ -64,25 +71,36 @@ __device__ __forceinline__ void group_transpose_reduce(A (&p)[U], unsigned gmask
 
 // PF == 0: gathered mat2 rows go global -> registers, double buffered.  PF > 0: they are staged through a per-group
 // shared-memory ring by cp.async exactly as in segment_reduce_kernel (PF sub-batches of U rows in flight).
-template <typename T, int VECW, int LPR, int VPL, int PF>
+// HV: vectors per head, a power of two; LPR * VPL is one head over the whole row (H = 1).
+template <typename T, int VECW, int LPR, int VPL, int PF, int HV = LPR * VPL>
 struct SddmmShape {
   static constexpr int NG = kThreads / LPR;
+  static constexpr int R = HV < LPR ? HV : LPR;                 // lanes that share a head's partial sums
+  static constexpr int HPJ = LPR / R;                           // heads in one vector layer j of the group
+  static constexpr int NP = HV < LPR ? VPL : VPL * LPR / HV;    // partials per lane and edge: heads it touches
+  static constexpr int NH = HPJ * NP;                           // heads the group holds
+  static_assert(HV <= LPR || HV % LPR == 0, "a head is whole vector layers or a power-of-two lane group");
   static constexpr int CW = LPR * VPL * VECW;
-  static constexpr int U0 = PF > 0 ? (VPL >= 4 ? 2 : 4) : ((VPL >= 4) ? 2 : (VPL == 2 ? 4 : 8));
+  // (several heads over several vector layers: half the sub-batch, for registers)
+  static constexpr int U0 = PF > 0 ? ((VPL >= 4 || (NH > 1 && VPL >= 2)) ? 2 : 4) : ((VPL >= 4) ? 2 : (VPL == 2 ? 4 : 8));
   static constexpr int U = (LPR < U0) ? LPR : U0;
   static constexpr int NS = PF + 1;
   static constexpr size_t smem_bytes = PF > 0 ? (size_t)NG * NS * U * CW * sizeof(T) : 0;
   static constexpr int max_blocks = (int)((227 * 1024) / (smem_bytes + 1024));
-  static constexpr int min_blocks = PF == 0 ? 2 : (max_blocks >= 3 ? 3 : (max_blocks >= 2 ? 2 : 1));
+  // (several heads: room for one result per head and the slot map of the collection below)
+  static constexpr int min_blocks = (PF == 0 || NH > 1) ? 2 : (max_blocks >= 3 ? 3 : (max_blocks >= 2 ? 2 : 1));
   static_assert(PF == 0 || PF * U <= LPR, "the prefetch distance must stay within one batch ahead");
 };
 
-template <typename T, int VECW, int LPR, int VPL, int PF>
-__global__ void __launch_bounds__(kThreads, (SddmmShape<T, VECW, LPR, VPL, PF>::min_blocks)) sddmm_coo_kernel(const SddmmParams p) {
+template <typename T, int VECW, int LPR, int VPL, int PF, int HV = LPR * VPL>
+__global__ void __launch_bounds__(kThreads, (SddmmShape<T, VECW, LPR, VPL, PF, HV>::min_blocks)) sddmm_coo_kernel(const SddmmParams p) {
   using A = typename AccOf<T>::type;
   using VecT = Vec<T, VECW>;
-  using SH = SddmmShape<T, VECW, LPR, VPL, PF>;
+  using SH = SddmmShape<T, VECW, LPR, VPL, PF, HV>;
   constexpr int NG = SH::NG, CW = SH::CW, U = SH::U, NS = SH::NS;
+  constexpr int R = SH::R, HPJ = SH::HPJ, NP = SH::NP, NH = SH::NH;
+  // after the butterfly over R lanes, value v = u * NP + q of the head group sits at lane (v / QV) * DV, slot v % QV
+  constexpr int NV = U * NP, QV = NV > R ? NV / R : 1, DV = NV < R ? R / NV : 1;
   extern __shared__ __align__(16) unsigned char sddmm_smem[];
 
   const int tid = threadIdx.x;
@@ -96,6 +114,7 @@ __global__ void __launch_bounds__(kThreads, (SddmmShape<T, VECW, LPR, VPL, PF>::
   const int64_t e_begin = ((int64_t)blockIdx.x * NG + g) * (int64_t)C;
   const int64_t e_end = min(e_begin + (int64_t)C, E);
   if (e_begin >= e_end) return;     // whole groups leave together: no block-level barrier below
+  const int64_t H = p.H;
 
   const T *__restrict__ mat1 = static_cast<const T *>(p.mat1);
   const T *__restrict__ mat2 = static_cast<const T *>(p.mat2);
@@ -182,6 +201,23 @@ __global__ void __launch_bounds__(kThreads, (SddmmShape<T, VECW, LPR, VPL, PF>::
   }
   int64_t last_row = -1;           // row_index of the edge left of the current batch (none yet: forces a load)
 
+  // The outputs this lane stores per batch: slot i is (edge k of the batch, head h); [H,E]: edge gl, head i; [E,H]:
+  // element gl + i * LPR of the batch's contiguous LPR * H outputs.  Per slot, 16 bits, two to a register: k (8 bits),
+  // and where the butterfly leaves (k, h): position v % QV (3 bits) of lane src (5 bits).
+  static_assert(NH <= 16 && QV <= 8, "slot fields");
+  unsigned slot2[(NH + 1) / 2];
+  if constexpr (NH > 1) {
+#pragma unroll
+    for (int i = 0; i < NH; ++i) {
+      const int k = p.head_major ? gl : (gl + i * LPR) / (int)H;
+      const int h = p.head_major ? i : gl + i * LPR - k * (int)H;
+      const int v = (k % U) * NP + h / HPJ;
+      const unsigned sl = (unsigned)((k << 8) | ((v % QV) << 5) | ((h % HPJ) * R + (v / QV) * DV));
+      slot2[i / 2] = (i % 2) ? (slot2[i / 2] | (sl << 16)) : sl;
+    }
+  }
+  auto slot = [&](int i) { return (int)((slot2[i / 2] >> ((i % 2) * 16)) & 0xffffu); };
+
   for (int64_t b = e_begin; b < e_end; b += LPR) {
     const bool has_next = b + LPR < e_end;
     int64_t nn_row = 0, nn_off1 = 0, nn_off2 = 0;
@@ -192,7 +228,9 @@ __global__ void __launch_bounds__(kThreads, (SddmmShape<T, VECW, LPR, VPL, PF>::
     const unsigned bmask = (__ballot_sync(gmask, my_row != left) >> gshift) & low_bits<LPR>();
     last_row = __shfl_sync(gmask, my_row, LPR - 1, LPR);
 
-    A mine = A(0);   // result of edge b + gl, collected from the sub-batches below
+    A mine[NH];      // results of this lane's output slots, collected from the sub-batches below
+#pragma unroll
+    for (int i = 0; i < NH; ++i) mine[i] = A(0);
 #pragma unroll
     for (int k0 = 0; k0 < LPR; k0 += U) {
       VecT vn[U][VPL];
@@ -217,25 +255,42 @@ __global__ void __launch_bounds__(kThreads, (SddmmShape<T, VECW, LPR, VPL, PF>::
         else if (has_next) load_v(vn, n_off2, 0);
       }
 
-      A part[U];
+      A part[NV];      // partial q of edge k0 + u at u * NP + q
       const unsigned sub = (bmask >> k0) & low_bits<U>();
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         if (sub != 0 && ((sub >> u) & 1u)) load_a(__shfl_sync(gmask, my_off1, k0 + u, LPR));
-        A s = A(0);
+        A s[NP];
+#pragma unroll
+        for (int q = 0; q < NP; ++q) s[q] = A(0);
 #pragma unroll
         for (int j = 0; j < VPL; ++j)
 #pragma unroll
-          for (int i = 0; i < VECW; ++i) s += a[j][i] * to_acc<T>(vc[u][j].v[i]);
-        part[u] = s;
+          for (int i = 0; i < VECW; ++i) s[HV < LPR ? j : j / (HV / LPR)] += a[j][i] * to_acc<T>(vc[u][j].v[i]);
+#pragma unroll
+        for (int q = 0; q < NP; ++q) part[u * NP + q] = s[q];
       }
-      if constexpr (LPR > 1) {
+      if constexpr (NH > 1) {
+        // head h is partial h / HPJ of the lanes [(h % HPJ) * R, +R); lane gl collects its slots of this sub-batch
+        group_transpose_reduce<NV, R, A>(part, gmask, gl);
+#pragma unroll
+        for (int i = 0; i < NH; ++i) {
+          const int src = slot(i) & 31;
+          A r = __shfl_sync(gmask, part[0], src, LPR);
+#pragma unroll
+          for (int q = 1; q < QV; ++q) {
+            const A t = __shfl_sync(gmask, part[q], src, LPR);
+            if (((slot(i) >> 5) & 7) == q) r = t;
+          }
+          if ((slot(i) >> 8) / U == k0 / U) mine[i] = r;
+        }
+      } else if constexpr (LPR > 1) {
         group_transpose_reduce<U, LPR, A>(part, gmask, gl);
         // value k sits in lanes [k*(LPR/U), (k+1)*(LPR/U)); lane gl wants edge gl = sub-batch gl/U, value gl%U
         const A r = __shfl_sync(gmask, part[0], (gl % U) * (LPR / U), LPR);
-        if (gl / U == k0 / U) mine = r;
+        if (gl / U == k0 / U) mine[0] = r;
       } else {
-        mine = part[0];
+        mine[0] = part[0];
       }
       if constexpr (PF == 0) {
 #pragma unroll
@@ -244,14 +299,27 @@ __global__ void __launch_bounds__(kThreads, (SddmmShape<T, VECW, LPR, VPL, PF>::
           for (int j = 0; j < VPL; ++j) vc[u][j] = vn[u][j];
       }
     }
-    if (b + gl < e_end) out[b + gl] = from_acc<T>(mine);
+    if constexpr (NH == 1) {
+      if (b + gl < e_end) out[b + gl] = from_acc<T>(mine[0]);
+    } else {
+#pragma unroll
+      for (int i = 0; i < NH; ++i) {
+        if (p.head_major) {
+          if (i < H && b + gl < e_end) out[i * E + b + gl] = from_acc<T>(mine[i]);
+        } else if (gl + i * LPR < LPR * H && b + (slot(i) >> 8) < e_end) {
+          out[b * H + gl + i * LPR] = from_acc<T>(mine[i]);
+        }
+      }
+    }
     my_row = n_row; my_off1 = n_off1; my_off2 = n_off2;
     n_row = nn_row; n_off1 = nn_off1; n_off2 = nn_off2;
   }
 }
 
-// Rows wider than a group can hold in registers (W > 32 lanes * 4 vectors): one warp per edge, columns in a loop.
-template <typename T>
+// Rows wider than a group can hold in registers (W > 32 lanes * 4 vectors), and heads without a lane mapping (not a
+// power-of-two number of whole vectors, or more than the group holds): one warp per edge, heads and columns in loops.
+// MH = false is the single-head (H = 1) instantiation.
+template <typename T, bool MH>
 __global__ void __launch_bounds__(kThreads) sddmm_coo_wide_kernel(const SddmmParams p) {
   using A = typename AccOf<T>::type;
   const int lane = threadIdx.x & 31;
@@ -260,14 +328,17 @@ __global__ void __launch_bounds__(kThreads) sddmm_coo_wide_kernel(const SddmmPar
   const T *__restrict__ mat1 = static_cast<const T *>(p.mat1);
   const T *__restrict__ mat2 = static_cast<const T *>(p.mat2);
   T *__restrict__ out = static_cast<T *>(p.out);
+  const int64_t H = MH ? p.H : 1, F = MH ? p.W / p.H : p.W;
   for (int64_t e = warp; e < p.E; e += n_warps) {
     const T *x = mat1 + p.row_index[e] * p.W;
     const T *y = mat2 + p.col_index[e] * p.W;
-    A s = A(0);
-    for (int64_t c = lane; c < p.W; c += 32) s += to_acc<T>(x[c]) * to_acc<T>(y[c]);
+    for (int64_t h = 0; h < H; ++h) {
+      A s = A(0);
+      for (int64_t c = h * F + lane; c < (h + 1) * F; c += 32) s += to_acc<T>(x[c]) * to_acc<T>(y[c]);
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    if (lane == 0) out[e] = from_acc<T>(s);
+      for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+      if (lane == 0) out[!MH ? e : p.head_major ? h * p.E + e : e * H + h] = from_acc<T>(s);
+    }
   }
 }
 

@@ -48,6 +48,12 @@ def _(src_index, dst_index, mat_1, mat_2):
     return mat_1.new_empty([src_index.shape[0]])
 
 
+@torch.library.register_fake("geot::sddmm_mh_impl")
+def _(src_index, dst_index, mat_1, mat_2, head_major):
+    E, H = src_index.shape[0], mat_1.shape[1]
+    return mat_1.new_empty([H, E] if head_major else [E, H])
+
+
 @torch.library.register_fake("geot::csr_gws_impl")
 def _(indptr, indices, weight, src):
     return src.new_empty([indptr.shape[0], src.shape[1]])

@@ -224,6 +224,14 @@ GEOT_API int geot_b200_sddmm_coo(const void *mat1, const int64_t *row_index, con
                         const int64_t *col_index, void *out, int64_t E, int64_t F, int dtype,
                         cudaStream_t stream);
 
+/* Multi-head SDDMM, the weight gradient of mh_spmm (one dot product per edge and head):
+ *     out[e, h] = < mat1[row_index[e], h, :], mat2[col_index[e], h, :] >   mat1 [N1,H,F], mat2 [N2,H,F]
+ * out is [E,H] (out_layout GEOT_W_EDGE_HEAD) or [H,E] (GEOT_W_HEAD_EDGE), the weight layouts of geot_b200_mh_spmm.
+ * All of `dtype`; bf16/fp16 accumulate in fp32 and round once.  No scratch, no sortedness requirement; a sorted
+ * row_index lets the kernel keep the mat1 row in registers.  H = 1 computes what geot_b200_sddmm_coo does. */
+GEOT_API int geot_b200_sddmm_mh(const void *mat1, const int64_t *row_index, const void *mat2, const int64_t *col_index,
+                       void *out, int64_t E, int64_t H, int64_t F, int dtype, int out_layout, cudaStream_t stream);
+
 /* CSR row pointer -> sorted COO row index (the inverse of geot::coo_to_csr): row_index[e] = r for
  * rowptr[r] <= e < rowptr[r+1].  rowptr has S+1 entries of 32 or 64 bits (rowptr_bits).  Lets the CSR entry
  * point csr_gws (csrc/csr_gws.cpp:24-35, csr_gws_cuda.cu) run on the same kernels. */
