@@ -29,6 +29,7 @@ SYMBOLS = [
     "geot_b200_host_graph_create", "geot_b200_host_graph_reduce", "geot_b200_host_graph_last_transfer",
     "geot_b200_host_graph_destroy", "geot_b200_src_blocks_suggest", "geot_b200_src_blocks_bytes",
     "geot_b200_src_blocks_scratch_bytes", "geot_b200_src_blocks_build", "geot_b200_src_blocks_workspace_bytes",
+    "geot_b200_segment_softmax_workspace_bytes", "geot_b200_segment_softmax", "geot_b200_segment_softmax_backward",
 ]
 
 
@@ -100,6 +101,11 @@ def lib() -> ctypes.CDLL:
                                         ctypes.POINTER(GeotPlan), vp, sz, vp]
         L.geot_b200_sddmm_coo.argtypes = [vp, vp, vp, vp, vp, i64, i64, ci, vp]
         L.geot_b200_sddmm_mh.argtypes = [vp, vp, vp, vp, vp, i64, i64, i64, ci, ci, vp]
+        L.geot_b200_segment_softmax_workspace_bytes.restype = sz
+        L.geot_b200_segment_softmax_workspace_bytes.argtypes = [i64, i64, ci]
+        L.geot_b200_segment_softmax.argtypes = [vp, vp, vp, i64, i64, ci, ctypes.POINTER(GeotPlan), vp, sz, vp]
+        L.geot_b200_segment_softmax_backward.argtypes = [vp, vp, vp, vp, i64, i64, ci, ctypes.POINTER(GeotPlan), vp, sz,
+                                                         vp]
         L.geot_b200_csr_to_coo.argtypes = [vp, ci, i64, i64, vp, vp]
         L.geot_b200_permute_edges.argtypes = [vp, vp, vp, i64, i64, vp]
         L.geot_b200_segment_reduce_host.argtypes = [vp, i64, vp, vp, vp, vp, i64, i64, i64, i64, ci, ci, ci]
@@ -254,6 +260,34 @@ def sddmm_mh(mat1, row_index, mat2, col_index, head_major=False):
     check(lib().geot_b200_sddmm_mh(_ptr(mat1), _ptr(row_index), _ptr(mat2), _ptr(col_index), _ptr(out), E, H, F,
                                    DTYPE[mat1.dtype], W_HEAD_EDGE if head_major else W_EDGE_HEAD, _stream()), "sddmm_mh")
     return out
+
+
+def _softmax_workspace(E, H, dtype, device):
+    n = lib().geot_b200_segment_softmax_workspace_bytes(E, H, DTYPE[dtype])
+    return torch.empty(n, dtype=torch.uint8, device=device), n
+
+
+def segment_softmax(src, dst_index, plan: DevicePlan = None):
+    """Softmax of src [E] / [E, H] over the edges of each dst row (dst_index sorted) through geot_b200_segment_softmax."""
+    E, H = dst_index.numel(), src[0].numel() if src.numel() else 1
+    plan = plan if plan is not None else DevicePlan(dst_index)
+    out = torch.empty_like(src)
+    ws, n = _softmax_workspace(E, H, src.dtype, src.device)
+    check(lib().geot_b200_segment_softmax(_ptr(src), _ptr(dst_index), _ptr(out), E, H, DTYPE[src.dtype],
+                                          ctypes.byref(plan.c), _ptr(ws), n, _stream()), "segment_softmax")
+    return out
+
+
+def segment_softmax_backward(out, grad_out, dst_index, plan: DevicePlan = None):
+    """grad_src = out * (grad_out - sum over the row of out * grad_out) through geot_b200_segment_softmax_backward."""
+    E, H = dst_index.numel(), out[0].numel() if out.numel() else 1
+    plan = plan if plan is not None else DevicePlan(dst_index)
+    grad_src = torch.empty_like(out)
+    ws, n = _softmax_workspace(E, H, out.dtype, out.device)
+    check(lib().geot_b200_segment_softmax_backward(_ptr(out), _ptr(grad_out), _ptr(dst_index), _ptr(grad_src), E, H,
+                                                   DTYPE[out.dtype], ctypes.byref(plan.c), _ptr(ws), n, _stream()),
+          "segment_softmax_backward")
+    return grad_src
 
 
 def csr_to_coo(rowptr, E):

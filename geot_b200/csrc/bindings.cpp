@@ -420,6 +420,66 @@ at::Tensor sddmm_mh_impl(at::Tensor src_index, at::Tensor dst_index, at::Tensor 
   return out;
 }
 
+// ---- segment softmax -------------------------------------------------------------------------------------
+// geot::segment_softmax / geot::segment_softmax_backward: src / out / grad [E] or [E, H] over a sorted int64 index [E].
+// The plan comes from the cache (no sync after the first call on a graph); an index it reports unsorted is refused.
+void check_softmax_operand(const at::Tensor &t, const at::Tensor &index, const char *what, const char *name) {
+  TORCH_CHECK(t.is_cuda(), "geot::", what, ": ", name, " must be a CUDA tensor (this build has no CPU path)");
+  TORCH_CHECK(t.dim() == 1 || t.dim() == 2, "geot::", what, ": ", name, " must be [E] or [E, H]");
+  TORCH_CHECK(t.size(0) == index.size(0), "geot::", what, ": ", name, " must have one row per index entry");
+  TORCH_CHECK(t.device() == index.device(), "geot::", what, ": ", name, " and index must be on the same device");
+}
+
+geot_plan_t softmax_plan(const at::Tensor &index, const char *what, at::Tensor *keepalive) {
+  geot_plan_t plan = get_plan(index, keepalive);
+  TORCH_CHECK(plan.is_sorted, "geot::", what, ": index must be sorted (non-decreasing)");
+  return plan;
+}
+
+at::Tensor segment_softmax_impl(at::Tensor src, at::Tensor index) {
+  check_index(index, "index");
+  TORCH_CHECK(index.dim() == 1, "geot::segment_softmax: index must be 1 dimensional");
+  check_softmax_operand(src, index, "segment_softmax", "src");
+  const int dtype = dtype_enum(src);
+  c10::cuda::CUDAGuard guard(src.device());
+  const at::Tensor x = src.contiguous(), idx = index.contiguous();
+  at::Tensor out = at::empty_like(x);
+  const int64_t E = idx.numel(), H = E > 0 ? x.numel() / E : 0;
+  if (E == 0 || H == 0) return out;
+  at::Tensor plan_buf;
+  const geot_plan_t plan = softmax_plan(idx, "segment_softmax", &plan_buf);
+  const size_t ws_bytes = geot_b200_segment_softmax_workspace_bytes(E, H, dtype);
+  at::Tensor ws = at::empty({(int64_t)ws_bytes}, x.options().dtype(at::kByte));
+  check_status(geot_b200_segment_softmax(x.data_ptr(), idx.data_ptr<int64_t>(), out.data_ptr(), E, H, dtype, &plan,
+                                         ws.data_ptr(), ws_bytes, at::cuda::getCurrentCUDAStream()),
+               "segment_softmax");
+  return out;
+}
+
+at::Tensor segment_softmax_backward_impl(at::Tensor out, at::Tensor grad_out, at::Tensor index) {
+  check_index(index, "index");
+  TORCH_CHECK(index.dim() == 1, "geot::segment_softmax_backward: index must be 1 dimensional");
+  check_softmax_operand(out, index, "segment_softmax_backward", "out");
+  check_softmax_operand(grad_out, index, "segment_softmax_backward", "grad_out");
+  TORCH_CHECK(out.sizes() == grad_out.sizes(), "geot::segment_softmax_backward: out and grad_out must have the same shape");
+  TORCH_CHECK(out.scalar_type() == grad_out.scalar_type(), "geot::segment_softmax_backward: out and grad_out must have the same dtype");
+  const int dtype = dtype_enum(out);
+  c10::cuda::CUDAGuard guard(out.device());
+  const at::Tensor y = out.contiguous(), g = grad_out.contiguous(), idx = index.contiguous();
+  at::Tensor grad_src = at::empty_like(y);
+  const int64_t E = idx.numel(), H = E > 0 ? y.numel() / E : 0;
+  if (E == 0 || H == 0) return grad_src;
+  at::Tensor plan_buf;
+  const geot_plan_t plan = softmax_plan(idx, "segment_softmax_backward", &plan_buf);
+  const size_t ws_bytes = geot_b200_segment_softmax_workspace_bytes(E, H, dtype);
+  at::Tensor ws = at::empty({(int64_t)ws_bytes}, y.options().dtype(at::kByte));
+  check_status(geot_b200_segment_softmax_backward(y.data_ptr(), g.data_ptr(), idx.data_ptr<int64_t>(), grad_src.data_ptr(),
+                                                  E, H, dtype, &plan, ws.data_ptr(), ws_bytes,
+                                                  at::cuda::getCurrentCUDAStream()),
+               "segment_softmax_backward");
+  return grad_src;
+}
+
 // ---- CSR entry point ------------------------------------------------------------------------------------
 // Cache of the COO row index expanded from a CSR row pointer, keyed like the plans (storage + version).
 struct CsrEntry {
@@ -521,6 +581,8 @@ TORCH_LIBRARY_FRAGMENT(geot, m) {
   m.def("format_preprocess(Tensor dst_index) -> (Tensor, Tensor)");
   m.def("plan_shards(Tensor dst_index, int parts) -> Tensor");
   m.def("sddmm_mh_impl(Tensor src_index, Tensor dst_index, Tensor mat_1, Tensor mat_2, bool head_major) -> Tensor");
+  m.def("segment_softmax(Tensor src, Tensor index) -> Tensor");
+  m.def("segment_softmax_backward(Tensor out, Tensor grad_out, Tensor index) -> Tensor");
   m.def("clear_plan_cache() -> ()", []() { clear_plan_cache(); });
   m.def("abi_version() -> int", []() { return (int64_t)geot_b200_version(); });
 }
@@ -538,4 +600,6 @@ TORCH_LIBRARY_IMPL(geot, CUDA, m) {
   m.impl("format_preprocess", format_preprocess);
   m.impl("plan_shards", plan_shards);
   m.impl("sddmm_mh_impl", sddmm_mh_impl);
+  m.impl("segment_softmax", segment_softmax_impl);
+  m.impl("segment_softmax_backward", segment_softmax_backward_impl);
 }

@@ -54,6 +54,16 @@ def _(src_index, dst_index, mat_1, mat_2, head_major):
     return mat_1.new_empty([H, E] if head_major else [E, H])
 
 
+@torch.library.register_fake("geot::segment_softmax")
+def _(src, index):
+    return torch.empty_like(src, memory_format=torch.contiguous_format)
+
+
+@torch.library.register_fake("geot::segment_softmax_backward")
+def _(out, grad_out, index):
+    return torch.empty_like(out, memory_format=torch.contiguous_format)
+
+
 @torch.library.register_fake("geot::csr_gws_impl")
 def _(indptr, indices, weight, src):
     return src.new_empty([indptr.shape[0], src.shape[1]])

@@ -11,6 +11,8 @@ PyG / torch_sparse are not part of this build, so the same math is restated on p
   ``format_preprocess`` plan are computed once per graph.
 * GraphSAGE layer (``models/conv/sageconv.py:122-154``, ``aggr="sum"`` as ``models/graphsage.py:48`` sets it):
   ``out = lin_l(sum_j x_j) + lin_r(x)`` -- one ``gather_scatter`` per layer.
+* GAT layer (PyG ``GATConv`` without dropout): the attention softmax is ``segment_softmax``, the weighted
+  aggregation ``mh_spmm`` -- both deterministic kernels of this library, both differentiable.
 * Stack (``models/basicgnn.py:216-264``): ``conv -> ReLU`` for every layer but the last; dropout p = 0.
 
 The dense ``lin`` layers are cuBLAS GEMMs through ``torch.nn.Linear`` (library code, not part of the hot
@@ -25,6 +27,8 @@ from torch import nn
 
 from .gather_scatter import gather_scatter
 from .gather_weight_scatter import gather_weight_scatter
+from .mh_spmm import mh_spmm
+from .softmax import segment_softmax
 
 
 def add_self_loops(src_index: torch.Tensor, dst_index: torch.Tensor, num_nodes: int,
@@ -85,6 +89,38 @@ class SAGEConv(nn.Module):
     def forward(self, x, src_index, dst_index, reduce: str = "sum"):
         agg = _pad_rows(gather_scatter(src_index, dst_index, x, reduce), x.shape[0])
         return self.lin_l(agg) + self.lin_r(x)
+
+
+class GATConv(nn.Module):
+    """PyG's ``GATConv`` math without dropout, on a dst-sorted edge list (the caller adds self loops with
+    ``add_self_loops``): ``h = lin(x)`` as ``[N, H, F]``; per edge and head
+    ``alpha = softmax_row(leaky_relu(<h[src], att_src> + <h[dst], att_dst>))`` (``segment_softmax``); the aggregation
+    ``out[dst] = sum alpha * h[src]`` is ``mh_spmm``; the heads are concatenated (``concat``) or averaged, then ``bias``
+    is added.  Differentiable end to end."""
+
+    def __init__(self, in_channels: int, out_channels: int, heads: int = 1, concat: bool = True,
+                 negative_slope: float = 0.2, bias: bool = True):
+        super().__init__()
+        self.heads, self.out_channels, self.concat, self.negative_slope = heads, out_channels, concat, negative_slope
+        self.lin = nn.Linear(in_channels, heads * out_channels, bias=False)
+        self.att_src = nn.Parameter(torch.empty(1, heads, out_channels))
+        self.att_dst = nn.Parameter(torch.empty(1, heads, out_channels))
+        self.bias = nn.Parameter(torch.zeros(heads * out_channels if concat else out_channels)) if bias else None
+        nn.init.xavier_uniform_(self.lin.weight)
+        nn.init.xavier_uniform_(self.att_src)
+        nn.init.xavier_uniform_(self.att_dst)
+
+    def forward(self, x, src_index, dst_index):
+        N, H, F = x.shape[0], self.heads, self.out_channels
+        h = self.lin(x).view(N, H, F)
+        a_src = (h * self.att_src).sum(-1)
+        a_dst = (h * self.att_dst).sum(-1)
+        logits = torch.nn.functional.leaky_relu(a_src.index_select(0, src_index) + a_dst.index_select(0, dst_index),
+                                                self.negative_slope)
+        alpha = segment_softmax(logits, dst_index)
+        out = _pad_rows(mh_spmm(src_index, dst_index, alpha, h), N)
+        out = out.reshape(N, H * F) if self.concat else out.mean(1)
+        return out + self.bias if self.bias is not None else out
 
 
 class _Stack(nn.Module):

@@ -232,6 +232,25 @@ GEOT_API int geot_b200_sddmm_coo(const void *mat1, const int64_t *row_index, con
 GEOT_API int geot_b200_sddmm_mh(const void *mat1, const int64_t *row_index, const void *mat2, const int64_t *col_index,
                        void *out, int64_t E, int64_t H, int64_t F, int dtype, int out_layout, cudaStream_t stream);
 
+/* Segment softmax over the edges of each dst row -- the attention weights of a GAT layer:
+ *     out[e, h] = exp(src[e, h] - m[r, h]) / sum_{e' : dst_index[e'] = r} exp(src[e', h] - m[r, h]),   r = dst_index[e]
+ * with m[r, h] the row's largest logit.  src / out [E, H] row-major, of `dtype`; dst_index [E] int64, non-decreasing
+ * (plan->is_sorted; the plan of dst_index from geot_b200_format_preprocess).  bf16/fp16/fp32 accumulate in fp32, fp64 in
+ * fp64, with the accurate exp and one IEEE division per element; special values per (row, head) as torch.softmax: a NaN
+ * or a +inf logit makes the row NaN, a row of -inf is NaN.  Edge-balanced (a hub row is cut over many CTAs), no
+ * atomics: the result is bit-reproducible.  Returns GEOT_ERR_EMPTY for E == 0 and GEOT_ERR_INVALID_ARG for an unsorted
+ * plan; workspace: geot_b200_segment_softmax_workspace_bytes (256-byte aligned). */
+GEOT_API size_t geot_b200_segment_softmax_workspace_bytes(int64_t E, int64_t H, int dtype);
+GEOT_API int geot_b200_segment_softmax(const void *src, const int64_t *dst_index, void *out, int64_t E, int64_t H,
+                              int dtype, const geot_plan_t *plan, void *workspace, size_t workspace_bytes,
+                              cudaStream_t stream);
+/* Its backward, from the forward's output:
+ *     grad_src[e, h] = out[e, h] * (grad_out[e, h] - sum_{e' : dst_index[e'] = r} out[e', h] * grad_out[e', h])
+ * Same operands, precision, partition, determinism, status codes and workspace as geot_b200_segment_softmax. */
+GEOT_API int geot_b200_segment_softmax_backward(const void *out, const void *grad_out, const int64_t *dst_index,
+                                       void *grad_src, int64_t E, int64_t H, int dtype, const geot_plan_t *plan,
+                                       void *workspace, size_t workspace_bytes, cudaStream_t stream);
+
 /* CSR row pointer -> sorted COO row index (the inverse of geot::coo_to_csr): row_index[e] = r for
  * rowptr[r] <= e < rowptr[r+1].  rowptr has S+1 entries of 32 or 64 bits (rowptr_bits).  Lets the CSR entry
  * point csr_gws (csrc/csr_gws.cpp:24-35, csr_gws_cuda.cu) run on the same kernels. */
