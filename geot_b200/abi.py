@@ -30,6 +30,7 @@ SYMBOLS = [
     "geot_b200_host_graph_destroy", "geot_b200_src_blocks_suggest", "geot_b200_src_blocks_bytes",
     "geot_b200_src_blocks_scratch_bytes", "geot_b200_src_blocks_build", "geot_b200_src_blocks_workspace_bytes",
     "geot_b200_segment_softmax_workspace_bytes", "geot_b200_segment_softmax", "geot_b200_segment_softmax_backward",
+    "geot_b200_gatv2_score", "geot_b200_gatv2_grad_workspace_bytes", "geot_b200_gatv2_grad",
 ]
 
 
@@ -106,6 +107,11 @@ def lib() -> ctypes.CDLL:
         L.geot_b200_segment_softmax.argtypes = [vp, vp, vp, i64, i64, ci, ctypes.POINTER(GeotPlan), vp, sz, vp]
         L.geot_b200_segment_softmax_backward.argtypes = [vp, vp, vp, vp, i64, i64, ci, ctypes.POINTER(GeotPlan), vp, sz,
                                                          vp]
+        L.geot_b200_gatv2_score.argtypes = [vp, vp, vp, vp, vp, vp, i64, i64, i64, ci, ctypes.POINTER(ctypes.c_double), vp]
+        L.geot_b200_gatv2_grad_workspace_bytes.restype = sz
+        L.geot_b200_gatv2_grad_workspace_bytes.argtypes = [i64, i64, i64, ci]
+        L.geot_b200_gatv2_grad.argtypes = [vp, vp, vp, vp, vp, vp, ctypes.POINTER(GeotPlan), i64, vp, vp, i64, i64, i64,
+                                           ci, ctypes.POINTER(ctypes.c_double), vp, sz, vp]
         L.geot_b200_csr_to_coo.argtypes = [vp, ci, i64, i64, vp, vp]
         L.geot_b200_permute_edges.argtypes = [vp, vp, vp, i64, i64, vp]
         L.geot_b200_segment_reduce_host.argtypes = [vp, i64, vp, vp, vp, vp, i64, i64, i64, i64, ci, ci, ci]
@@ -288,6 +294,35 @@ def segment_softmax_backward(out, grad_out, dst_index, plan: DevicePlan = None):
                                                    DTYPE[out.dtype], ctypes.byref(plan.c), _ptr(ws), n, _stream()),
           "segment_softmax_backward")
     return grad_src
+
+
+def gatv2_score(x_l, x_r, att, src_index, dst_index, negative_slope=0.2):
+    """[E, H] GATv2 scores sum_f att[h, f] * leaky_relu(x_l[src[e], h, f] + x_r[dst[e], h, f]) through
+    geot_b200_gatv2_score; x_l / x_r [N, H, F], att [H, F]."""
+    E, H, F = dst_index.numel(), x_l.shape[1], x_l.shape[2]
+    out = torch.empty(E, H, dtype=x_l.dtype, device=x_l.device)
+    check(lib().geot_b200_gatv2_score(_ptr(x_l), _ptr(x_r), _ptr(att), _ptr(src_index), _ptr(dst_index), _ptr(out), E, H,
+                                      F, DTYPE[x_l.dtype], ctypes.byref(ctypes.c_double(negative_slope)), _stream()),
+          "gatv2_score")
+    return out
+
+
+def gatv2_grad(x_row, x_gat, att, grad_score, row_index, gat_index, S_out, negative_slope=0.2, want_att=True,
+               plan: DevicePlan = None):
+    """One backward pass of the GATv2 score through geot_b200_gatv2_grad: (grad_row [S_out, H, F], grad_att [H, F] or
+    None); row_index sorted."""
+    E, H, F = row_index.numel(), x_row.shape[1], x_row.shape[2]
+    plan = plan if plan is not None else DevicePlan(row_index)
+    grad_row = torch.empty(S_out, H, F, dtype=x_row.dtype, device=x_row.device)
+    grad_att = torch.empty(H, F, dtype=x_row.dtype, device=x_row.device) if want_att else None
+    n = lib().geot_b200_gatv2_grad_workspace_bytes(E, H, F, DTYPE[x_row.dtype])
+    ws = torch.empty(n, dtype=torch.uint8, device=x_row.device)
+    check(lib().geot_b200_gatv2_grad(_ptr(x_row), _ptr(x_gat), _ptr(att), _ptr(grad_score), _ptr(row_index),
+                                     _ptr(gat_index), ctypes.byref(plan.c), S_out, _ptr(grad_row),
+                                     _ptr(grad_att) if want_att else None, E, H, F, DTYPE[x_row.dtype],
+                                     ctypes.byref(ctypes.c_double(negative_slope)),
+                                     _ptr(ws), n, _stream()), "gatv2_grad")
+    return grad_row, grad_att
 
 
 def csr_to_coo(rowptr, E):

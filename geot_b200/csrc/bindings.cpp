@@ -480,6 +480,105 @@ at::Tensor segment_softmax_backward_impl(at::Tensor out, at::Tensor grad_out, at
   return grad_src;
 }
 
+// ---- GATv2 attention score ---------------------------------------------------------------------------------
+// geot::gatv2_score: score[e, h] = sum_f att[h, f] * leaky_relu(x_l[src[e], h, f] + x_r[dst[e], h, f]), x_l [N_l, H, F],
+// x_r [N_r, H, F], att [H, F], dst_index sorted (the plan cache says so; an unsorted index is refused).
+void check_gatv2_operands(const at::Tensor &x_l, const at::Tensor &x_r, const at::Tensor &att, const at::Tensor &src_index,
+                          const at::Tensor &dst_index, const char *what) {
+  TORCH_CHECK(x_l.is_cuda() && x_r.is_cuda() && att.is_cuda(), "geot::", what,
+              ": x_l, x_r and att must be CUDA tensors (this build has no CPU path)");
+  check_index(src_index, "src_index");
+  check_index(dst_index, "dst_index");
+  TORCH_CHECK(src_index.dim() == 1 && dst_index.dim() == 1 && src_index.numel() == dst_index.numel(), "geot::", what,
+              ": src_index and dst_index must be 1 dimensional and of the same length");
+  TORCH_CHECK(x_l.dim() == 3 && x_r.dim() == 3 && x_l.size(1) == x_r.size(1) && x_l.size(2) == x_r.size(2), "geot::", what,
+              ": x_l and x_r must be [N, H, F] with the same H and F");
+  TORCH_CHECK(att.dim() == 2 && att.size(0) == x_l.size(1) && att.size(1) == x_l.size(2), "geot::", what, ": att must be [H, F]");
+  TORCH_CHECK(x_l.size(1) > 0 && x_l.size(2) > 0, "geot::", what, ": x_l and x_r must have at least one head and one feature");
+  TORCH_CHECK(x_l.scalar_type() == x_r.scalar_type() && att.scalar_type() == x_l.scalar_type(), "geot::", what,
+              ": x_l, x_r and att must have the same dtype");
+  const auto dev = x_l.device();
+  TORCH_CHECK(x_r.device() == dev && att.device() == dev && src_index.device() == dev && dst_index.device() == dev, "geot::",
+              what, ": all operands must be on the same device");
+}
+
+at::Tensor gatv2_score_impl(at::Tensor x_l, at::Tensor x_r, at::Tensor att, at::Tensor src_index, at::Tensor dst_index,
+                            double negative_slope) {
+  check_gatv2_operands(x_l, x_r, att, src_index, dst_index, "gatv2_score");
+  const int dtype = dtype_enum(x_l);
+  c10::cuda::CUDAGuard guard(x_l.device());
+  const at::Tensor xl = x_l.contiguous(), xr = x_r.contiguous(), a = att.contiguous();
+  const at::Tensor si = src_index.contiguous(), di = dst_index.contiguous();
+  const int64_t E = di.numel(), H = xl.size(1), F = xl.size(2);
+  at::Tensor out = at::empty({E, H}, xl.options());
+  if (E == 0) return out;
+  at::Tensor plan_buf;
+  softmax_plan(di, "gatv2_score", &plan_buf);        // cached: refuses an unsorted dst_index
+  check_status(geot_b200_gatv2_score(xl.data_ptr(), xr.data_ptr(), a.data_ptr(), si.data_ptr<int64_t>(), di.data_ptr<int64_t>(),
+                                     out.data_ptr(), E, H, F, dtype, &negative_slope, at::cuda::getCurrentCUDAStream()),
+               "gatv2_score");
+  return out;
+}
+
+// geot::gatv2_score_backward -> (grad_x_l, grad_x_r, grad_att); a gradient not asked for comes back as an empty tensor.
+// The dst pass (grad_x_r, grad_att) runs on the dst-sorted list; the src pass (grad_x_l) on the transposed list
+// t_perm / t_dst_index (= src_index[t_perm], sorted) / t_src_index (= dst_index[t_perm]) with the grads carried into that
+// order.  Both plans come from the plan cache.
+void gatv2_pass(const at::Tensor &x_row, const at::Tensor &x_gat, const at::Tensor &att, const at::Tensor &g,
+                const at::Tensor &row_index, const at::Tensor &gat_index, at::Tensor &grad_row, at::Tensor *grad_att,
+                double slope) {
+  at::Tensor plan_buf;
+  const geot_plan_t plan = softmax_plan(row_index, "gatv2_score_backward", &plan_buf);
+  const int64_t E = row_index.numel(), H = x_row.size(1), F = x_row.size(2);
+  const int dtype = dtype_enum(x_row);
+  const size_t ws_bytes = geot_b200_gatv2_grad_workspace_bytes(E, H, F, dtype);
+  at::Tensor ws = at::empty({(int64_t)ws_bytes}, x_row.options().dtype(at::kByte));
+  check_status(geot_b200_gatv2_grad(x_row.data_ptr(), x_gat.data_ptr(), att.data_ptr(), g.data_ptr(), row_index.data_ptr<int64_t>(),
+                                    gat_index.data_ptr<int64_t>(), &plan, grad_row.size(0), grad_row.data_ptr(),
+                                    grad_att ? grad_att->data_ptr() : nullptr, E, H, F, dtype, &slope, ws.data_ptr(), ws_bytes,
+                                    at::cuda::getCurrentCUDAStream()),
+               "gatv2_score_backward");
+}
+
+std::tuple<at::Tensor, at::Tensor, at::Tensor> gatv2_score_backward_impl(
+    at::Tensor grad, at::Tensor x_l, at::Tensor x_r, at::Tensor att, at::Tensor src_index, at::Tensor dst_index,
+    at::Tensor t_perm, at::Tensor t_dst_index, at::Tensor t_src_index, double negative_slope, bool need_x_l, bool need_x_r,
+    bool need_att) {
+  check_gatv2_operands(x_l, x_r, att, src_index, dst_index, "gatv2_score_backward");
+  const int64_t E = dst_index.numel(), H = x_l.size(1);
+  TORCH_CHECK(grad.dim() == 2 && grad.size(0) == E && grad.size(1) == H, "geot::gatv2_score_backward: grad must be [E, H]");
+  TORCH_CHECK(grad.scalar_type() == x_l.scalar_type() && grad.device() == x_l.device(),
+              "geot::gatv2_score_backward: grad must have the dtype and device of x_l");
+  c10::cuda::CUDAGuard guard(x_l.device());
+  const at::Tensor xl = x_l.contiguous(), xr = x_r.contiguous(), a = att.contiguous(), g = grad.contiguous();
+  at::Tensor gl = need_x_l ? at::empty_like(xl) : at::empty({0}, xl.options());
+  at::Tensor gr = need_x_r ? at::empty_like(xr) : at::empty({0}, xl.options());
+  at::Tensor ga = need_att ? at::empty_like(a) : at::empty({0}, xl.options());
+  if (E == 0) {            // no edge: every gradient is zero
+    gl.zero_(); gr.zero_(); ga.zero_();
+    return std::make_tuple(gl, gr, ga);
+  }
+  const at::Tensor si = src_index.contiguous(), di = dst_index.contiguous();
+  if (need_x_r || need_att) {
+    at::Tensor gr_buf = need_x_r ? gr : at::empty_like(xr);
+    gatv2_pass(xr, xl, a, g, di, si, gr_buf, need_att ? &ga : nullptr, negative_slope);
+  }
+  if (need_x_l) {
+    check_index(t_perm, "t_perm");
+    check_index(t_dst_index, "t_dst_index");
+    check_index(t_src_index, "t_src_index");
+    TORCH_CHECK(t_perm.numel() == E && t_dst_index.numel() == E && t_src_index.numel() == E,
+                "geot::gatv2_score_backward: the transposed edge list must have E entries");
+    const at::Tensor perm = t_perm.contiguous(), tdi = t_dst_index.contiguous(), tsi = t_src_index.contiguous();
+    at::Tensor gt = at::empty_like(g);
+    check_status(geot_b200_permute_edges(g.data_ptr(), perm.data_ptr<int64_t>(), gt.data_ptr(), E, H * (int64_t)g.element_size(),
+                                         at::cuda::getCurrentCUDAStream()),
+                 "gatv2_score_backward");
+    gatv2_pass(xl, xr, a, gt, tdi, tsi, gl, nullptr, negative_slope);
+  }
+  return std::make_tuple(gl, gr, ga);
+}
+
 // ---- CSR entry point ------------------------------------------------------------------------------------
 // Cache of the COO row index expanded from a CSR row pointer, keyed like the plans (storage + version).
 struct CsrEntry {
@@ -583,6 +682,10 @@ TORCH_LIBRARY_FRAGMENT(geot, m) {
   m.def("sddmm_mh_impl(Tensor src_index, Tensor dst_index, Tensor mat_1, Tensor mat_2, bool head_major) -> Tensor");
   m.def("segment_softmax(Tensor src, Tensor index) -> Tensor");
   m.def("segment_softmax_backward(Tensor out, Tensor grad_out, Tensor index) -> Tensor");
+  m.def("gatv2_score(Tensor x_l, Tensor x_r, Tensor att, Tensor src_index, Tensor dst_index, float negative_slope) -> Tensor");
+  m.def("gatv2_score_backward(Tensor grad, Tensor x_l, Tensor x_r, Tensor att, Tensor src_index, Tensor dst_index, "
+        "Tensor t_perm, Tensor t_dst_index, Tensor t_src_index, float negative_slope, bool need_x_l, bool need_x_r, "
+        "bool need_att) -> (Tensor, Tensor, Tensor)");
   m.def("clear_plan_cache() -> ()", []() { clear_plan_cache(); });
   m.def("abi_version() -> int", []() { return (int64_t)geot_b200_version(); });
 }
@@ -602,4 +705,6 @@ TORCH_LIBRARY_IMPL(geot, CUDA, m) {
   m.impl("sddmm_mh_impl", sddmm_mh_impl);
   m.impl("segment_softmax", segment_softmax_impl);
   m.impl("segment_softmax_backward", segment_softmax_backward_impl);
+  m.impl("gatv2_score", gatv2_score_impl);
+  m.impl("gatv2_score_backward", gatv2_score_backward_impl);
 }

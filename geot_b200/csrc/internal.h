@@ -39,3 +39,10 @@ int segment_reduce_impl(const void *src, const int64_t *src_index, const int64_t
                         int dtype, int reduce, int weight_layout, int sorted, const geot_plan_t *plan,
                         void *workspace, size_t workspace_bytes, cudaStream_t stream, const geot_reduce_opts_t *opts,
                         const Extra &ex);
+
+// The SDDMM launcher (sddmm.cu): out[e, h] = sum over a head's columns of mat1[row_index[e]] * mat2[col_index[e]], or
+// with att != null the GATv2 score att * leaky_relu(mat1 + mat2) of slope `slope`.  Arguments already validated.
+namespace geot {
+int sddmm(const void *mat1, const int64_t *row_index, const void *mat2, const int64_t *col_index, void *out, int64_t E,
+          int64_t H, int64_t F, int dtype, int head_major, cudaStream_t stream, const void *att, double slope);
+}  // namespace geot

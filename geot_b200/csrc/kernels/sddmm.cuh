@@ -25,6 +25,10 @@
 //     lane bits only and a lane keeps one partial per vector it holds (each of its VPL vectors is in another head);
 //     the results are then gathered so that the LPR * H outputs of a batch leave in coalesced stores, as [E,H] (the
 //     H results of an edge contiguous) or [H,E] (the edges of a head contiguous).
+//   * OP: the elementwise step before the reduction over a head's columns.  SDDMM_DOT (the default) is a * b;
+//     SDDMM_GATV2 is att[c] * leaky_relu(a + b) -- the GATv2 attention score with mat1 = x_r by dst, mat2 = x_l by src
+//     (gatv2.cu).  a + b is formed in the accumulator, then the slope, then the product with att; one rounding on the
+//     store.  A lane holds the same columns for every edge, so its att values are loaded once.
 #pragma once
 #include "segment_reduce.cuh"
 
@@ -42,6 +46,17 @@ struct SddmmParams {
   int head_major;
   int chunk_edges;
 };
+
+// gatv2_score_kernel: the same operands, plus
+struct Gatv2ScoreParams : SddmmParams {
+  const void *att;              // [H, F] = [W], of the operands' type
+  double slope;                 // leaky_relu negative slope
+};
+
+enum : int { SDDMM_DOT = 0, SDDMM_GATV2 = 1 };
+
+// leaky_relu as torch computes it: u > 0 ? u : u * slope (NaN goes through the product)
+template <typename A> __device__ __forceinline__ A leaky(A u, A slope) { return u > A(0) ? u : u * slope; }
 
 // Transposing butterfly over the low log2(LPR) lane bits: p[0..U) per lane in.  On return, with U <= LPR, p[0] of lane
 // gl holds the sum over its LPR lanes of value ((gl % LPR) / (LPR / U)); with U > LPR, p[0 .. U/LPR) hold values
@@ -89,11 +104,14 @@ struct SddmmShape {
   static constexpr int max_blocks = (int)((227 * 1024) / (smem_bytes + 1024));
   // (several heads: room for one result per head and the slot map of the collection below)
   static constexpr int min_blocks = (PF == 0 || NH > 1) ? 2 : (max_blocks >= 3 ? 3 : (max_blocks >= 2 ? 2 : 1));
+  // SDDMM_GATV2 holds the lane's att columns too: one CTA fewer per SM, so that no shape spills
+  static constexpr int min_blocks_of(int op) { return op == 0 ? min_blocks : min_blocks - 1; }
   static_assert(PF == 0 || PF * U <= LPR, "the prefetch distance must stay within one batch ahead");
 };
 
-template <typename T, int VECW, int LPR, int VPL, int PF, int HV = LPR * VPL>
-__global__ void __launch_bounds__(kThreads, (SddmmShape<T, VECW, LPR, VPL, PF, HV>::min_blocks)) sddmm_coo_kernel(const SddmmParams p) {
+// P: SddmmParams, or Gatv2ScoreParams for OP = SDDMM_GATV2.
+template <typename T, int VECW, int LPR, int VPL, int PF, int HV = LPR * VPL, int OP = SDDMM_DOT, typename P = SddmmParams>
+__global__ void __launch_bounds__(kThreads, (SddmmShape<T, VECW, LPR, VPL, PF, HV>::min_blocks_of(OP))) sddmm_coo_kernel(const P p) {
   using A = typename AccOf<T>::type;
   using VecT = Vec<T, VECW>;
   using SH = SddmmShape<T, VECW, LPR, VPL, PF, HV>;
@@ -133,6 +151,17 @@ __global__ void __launch_bounds__(kThreads, (SddmmShape<T, VECW, LPR, VPL, PF, H
   }
   const char *m1 = reinterpret_cast<const char *>(mat1);
   const char *m2 = reinterpret_cast<const char *>(mat2);
+  [[maybe_unused]] A att[OP == SDDMM_GATV2 ? VPL : 1][OP == SDDMM_GATV2 ? VECW : 1];
+  [[maybe_unused]] A slope = A(0);
+  if constexpr (OP == SDDMM_GATV2) {
+    slope = A(p.slope);
+#pragma unroll
+    for (int j = 0; j < VPL; ++j) {
+      const VecT v = *reinterpret_cast<const VecT *>(static_cast<const char *>(p.att) + col_b[j]);
+#pragma unroll
+      for (int i = 0; i < VECW; ++i) att[j][i] = to_acc<T>(v.v[i]);
+    }
+  }
 
   T *ring = nullptr;      // this group's ring; lane piece j of row r at r*CW + (j*LPR + gl)*VECW
   uint32_t ring_s = 0;
@@ -266,7 +295,14 @@ __global__ void __launch_bounds__(kThreads, (SddmmShape<T, VECW, LPR, VPL, PF, H
 #pragma unroll
         for (int j = 0; j < VPL; ++j)
 #pragma unroll
-          for (int i = 0; i < VECW; ++i) s[HV < LPR ? j : j / (HV / LPR)] += a[j][i] * to_acc<T>(vc[u][j].v[i]);
+          for (int i = 0; i < VECW; ++i) {
+            if constexpr (OP == SDDMM_GATV2) {
+              // lanes past the row end hold no columns: nothing, not att * leaky of column 0
+              if (col_ok[j]) s[HV < LPR ? j : j / (HV / LPR)] += att[j][i] * leaky(a[j][i] + to_acc<T>(vc[u][j].v[i]), slope);
+            } else {
+              s[HV < LPR ? j : j / (HV / LPR)] += a[j][i] * to_acc<T>(vc[u][j].v[i]);
+            }
+          }
 #pragma unroll
         for (int q = 0; q < NP; ++q) part[u * NP + q] = s[q];
       }
@@ -319,8 +355,8 @@ __global__ void __launch_bounds__(kThreads, (SddmmShape<T, VECW, LPR, VPL, PF, H
 // Rows wider than a group can hold in registers (W > 32 lanes * 4 vectors), and heads without a lane mapping (not a
 // power-of-two number of whole vectors, or more than the group holds): one warp per edge, heads and columns in loops.
 // MH = false is the single-head (H = 1) instantiation.
-template <typename T, bool MH>
-__global__ void __launch_bounds__(kThreads) sddmm_coo_wide_kernel(const SddmmParams p) {
+template <typename T, bool MH, int OP = SDDMM_DOT, typename P = SddmmParams>
+__global__ void __launch_bounds__(kThreads) sddmm_coo_wide_kernel(const P p) {
   using A = typename AccOf<T>::type;
   const int lane = threadIdx.x & 31;
   const int64_t warp = ((int64_t)blockIdx.x * kThreads + threadIdx.x) >> 5;
@@ -334,7 +370,14 @@ __global__ void __launch_bounds__(kThreads) sddmm_coo_wide_kernel(const SddmmPar
     const T *y = mat2 + p.col_index[e] * p.W;
     for (int64_t h = 0; h < H; ++h) {
       A s = A(0);
-      for (int64_t c = h * F + lane; c < (h + 1) * F; c += 32) s += to_acc<T>(x[c]) * to_acc<T>(y[c]);
+      if constexpr (OP == SDDMM_GATV2) {
+        const T *att = static_cast<const T *>(p.att);
+        const A slope = A(p.slope);
+        for (int64_t c = h * F + lane; c < (h + 1) * F; c += 32)
+          s += to_acc<T>(att[c]) * leaky(to_acc<T>(x[c]) + to_acc<T>(y[c]), slope);
+      } else {
+        for (int64_t c = h * F + lane; c < (h + 1) * F; c += 32) s += to_acc<T>(x[c]) * to_acc<T>(y[c]);
+      }
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
       if (lane == 0) out[!MH ? e : p.head_major ? h * p.E + e : e * H + h] = from_acc<T>(s);

@@ -64,6 +64,19 @@ def _(out, grad_out, index):
     return torch.empty_like(out, memory_format=torch.contiguous_format)
 
 
+@torch.library.register_fake("geot::gatv2_score")
+def _(x_l, x_r, att, src_index, dst_index, negative_slope):
+    return x_l.new_empty([dst_index.shape[0], x_l.shape[1]])
+
+
+@torch.library.register_fake("geot::gatv2_score_backward")
+def _(grad, x_l, x_r, att, src_index, dst_index, t_perm, t_dst_index, t_src_index, negative_slope, need_x_l, need_x_r,
+      need_att):
+    def like(t, need):
+        return t.new_empty(t.shape) if need else t.new_empty([0])
+    return like(x_l, need_x_l), like(x_r, need_x_r), like(att, need_att)
+
+
 @torch.library.register_fake("geot::csr_gws_impl")
 def _(indptr, indices, weight, src):
     return src.new_empty([indptr.shape[0], src.shape[1]])

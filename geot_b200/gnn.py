@@ -13,6 +13,8 @@ PyG / torch_sparse are not part of this build, so the same math is restated on p
   ``out = lin_l(sum_j x_j) + lin_r(x)`` -- one ``gather_scatter`` per layer.
 * GAT layer (PyG ``GATConv`` without dropout): the attention softmax is ``segment_softmax``, the weighted
   aggregation ``mh_spmm`` -- both deterministic kernels of this library, both differentiable.
+* GATv2 layer (PyG ``GATv2Conv``, ``share_weights=False``, without dropout and edge features): the attention score is
+  the fused ``gatv2_score``, then ``segment_softmax`` and ``mh_spmm``.
 * Stack (``models/basicgnn.py:216-264``): ``conv -> ReLU`` for every layer but the last; dropout p = 0.
 
 The dense ``lin`` layers are cuBLAS GEMMs through ``torch.nn.Linear`` (library code, not part of the hot
@@ -29,6 +31,7 @@ from .gather_scatter import gather_scatter
 from .gather_weight_scatter import gather_weight_scatter
 from .mh_spmm import mh_spmm
 from .softmax import segment_softmax
+from .gatv2 import gatv2_score
 
 
 def add_self_loops(src_index: torch.Tensor, dst_index: torch.Tensor, num_nodes: int,
@@ -119,6 +122,48 @@ class GATConv(nn.Module):
                                                 self.negative_slope)
         alpha = segment_softmax(logits, dst_index)
         out = _pad_rows(mh_spmm(src_index, dst_index, alpha, h), N)
+        out = out.reshape(N, H * F) if self.concat else out.mean(1)
+        return out + self.bias if self.bias is not None else out
+
+
+class GATv2Conv(nn.Module):
+    """PyG's ``GATv2Conv`` math on a dst-sorted edge list (the caller adds self loops with ``add_self_loops``):
+    ``x_l = lin_l(x)`` and ``x_r = lin_r(x)`` as ``[N, H, F]``; per edge and head
+    ``score = sum_f att[h, f] * leaky_relu(x_l[src, h, f] + x_r[dst, h, f])`` (the fused ``gatv2_score``),
+    ``alpha = softmax_row(score)`` (``segment_softmax``); the aggregation ``out[dst] = sum alpha * x_l[src]`` is
+    ``mh_spmm``; the heads are concatenated (``concat``) or averaged, then ``bias`` is added.  ``lin_l``, ``lin_r`` and
+    ``att`` get PyG's glorot initialisation, ``lin_l`` / ``lin_r`` carry a bias when ``bias`` is set, and the output bias
+    starts at zero, as in PyG.  Left out of PyG's options: ``share_weights`` (always separate ``lin_l`` / ``lin_r``),
+    ``edge_dim``, attention ``dropout``, ``add_self_loops`` (done by the caller) and ``residual``.  Differentiable end to
+    end; no ``[E, H * F]`` tensor is materialised."""
+
+    def __init__(self, in_channels: int, out_channels: int, heads: int = 1, concat: bool = True,
+                 negative_slope: float = 0.2, bias: bool = True):
+        super().__init__()
+        self.heads, self.out_channels, self.concat, self.negative_slope = heads, out_channels, concat, negative_slope
+        self.lin_l = nn.Linear(in_channels, heads * out_channels, bias=bias)
+        self.lin_r = nn.Linear(in_channels, heads * out_channels, bias=bias)
+        self.att = nn.Parameter(torch.empty(1, heads, out_channels))
+        self.bias = nn.Parameter(torch.zeros(heads * out_channels if concat else out_channels)) if bias else None
+        self.reset_parameters()
+
+    def reset_parameters(self):
+        # PyG: Linear(weight_initializer="glorot") with zero biases, glorot(att), zeros(bias)
+        for lin in (self.lin_l, self.lin_r):
+            nn.init.xavier_uniform_(lin.weight)
+            if lin.bias is not None:
+                nn.init.zeros_(lin.bias)
+        nn.init.xavier_uniform_(self.att)
+        if self.bias is not None:
+            nn.init.zeros_(self.bias)
+
+    def forward(self, x, src_index, dst_index):
+        N, H, F = x.shape[0], self.heads, self.out_channels
+        x_l = self.lin_l(x).view(N, H, F)
+        x_r = self.lin_r(x).view(N, H, F)
+        score = gatv2_score(x_l, x_r, self.att, src_index, dst_index, self.negative_slope)
+        alpha = segment_softmax(score, dst_index)
+        out = _pad_rows(mh_spmm(src_index, dst_index, alpha, x_l), N)
         out = out.reshape(N, H * F) if self.concat else out.mean(1)
         return out + self.bias if self.bias is not None else out
 

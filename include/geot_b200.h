@@ -251,6 +251,32 @@ GEOT_API int geot_b200_segment_softmax_backward(const void *out, const void *gra
                                        void *grad_src, int64_t E, int64_t H, int dtype, const geot_plan_t *plan,
                                        void *workspace, size_t workspace_bytes, cudaStream_t stream);
 
+/* GATv2 attention score (PyG GATv2Conv, share_weights = False) of every edge and head:
+ *     score[e, h] = sum_f att[h, f] * leaky_relu(x_l[src_index[e], h, f] + x_r[dst_index[e], h, f])
+ * leaky_relu(u) = u > 0 ? u : slope * u, slope = *negative_slope (host memory, read before the call returns; only
+ * integers, sizes and pointers cross this ABI).  x_l [N_l, H, F], x_r [N_r, H, F], att [H, F], out [E, H], all of
+ * `dtype`; bf16/fp16/fp32 accumulate in fp32, fp64 in fp64: the sum x_l + x_r is formed in the accumulator, then the
+ * slope, then the product with att; one rounding on the store.  No scratch; a sorted dst_index lets the kernel keep the
+ * x_r row in registers while dst repeats.  Returns GEOT_ERR_EMPTY for E == 0. */
+GEOT_API int geot_b200_gatv2_score(const void *x_l, const void *x_r, const void *att, const int64_t *src_index,
+                          const int64_t *dst_index, void *out, int64_t E, int64_t H, int64_t F, int dtype,
+                          const double *negative_slope, cudaStream_t stream);
+/* Its backward, one pass per node operand.  For g = grad_score [E, H] in the edge order of row_index:
+ *     grad_row[r, h, f] = att[h, f] * sum_{e : row_index[e] = r} g[e, h] * leaky'(x_row[r, h, f] + x_gat[gat_index[e], h, f])
+ *     grad_att[h, f]    = sum_e g[e, h] * leaky_relu(x_row[row_index[e], h, f] + x_gat[gat_index[e], h, f])
+ * with leaky'(u) = u > 0 ? 1 : slope (torch's leaky_relu_backward).  The dst pass is row = x_r, row_index =
+ * dst_index, gat = x_l by src_index; the src pass runs on the src-sorted (transposed) edge list with row = x_l and the
+ * grads carried into that order (geot_b200_permute_edges).  row_index is non-decreasing: plan is its plan
+ * (geot_b200_format_preprocess), with plan->max_row < S_out.  grad_row [S_out, H, F] is fully written (rows without
+ * edges are 0); grad_att [H, F] may be NULL.  Same precision as the score; edge-balanced, no atomics: bit-reproducible.
+ * Returns GEOT_ERR_EMPTY for E == 0, GEOT_ERR_INVALID_ARG for an unsorted plan, a plan of another index or a plan
+ * whose largest index is >= S_out; workspace: geot_b200_gatv2_grad_workspace_bytes (256-byte aligned). */
+GEOT_API size_t geot_b200_gatv2_grad_workspace_bytes(int64_t E, int64_t H, int64_t F, int dtype);
+GEOT_API int geot_b200_gatv2_grad(const void *x_row, const void *x_gat, const void *att, const void *grad_score,
+                         const int64_t *row_index, const int64_t *gat_index, const geot_plan_t *plan, int64_t S_out,
+                         void *grad_row, void *grad_att, int64_t E, int64_t H, int64_t F, int dtype,
+                         const double *negative_slope, void *workspace, size_t workspace_bytes, cudaStream_t stream);
+
 /* CSR row pointer -> sorted COO row index (the inverse of geot::coo_to_csr): row_index[e] = r for
  * rowptr[r] <= e < rowptr[r+1].  rowptr has S+1 entries of 32 or 64 bits (rowptr_bits).  Lets the CSR entry
  * point csr_gws (csrc/csr_gws.cpp:24-35, csr_gws_cuda.cu) run on the same kernels. */

@@ -35,7 +35,7 @@ want = ["segment_reduce_kernel<float, 4, 32, 1, 0, 1, 35>", "segment_reduce_kern
         "segment_reduce_kernel<float, 4, 16, 1, 0, 0, 35>", "segment_reduce_kernel<float, 4, 32, 2, 0, 0, 35>",
         "segment_reduce_kernel<float, 4, 32, 2, 0, 1, 35>", "segment_reduce_kernel<float, 4, 16, 1, 0, 0, 39>",
         "segment_reduce_kernel<__nv_bfloat16, 8, 32, 1, 0, 2, 3>", "segment_fixup_kernel<float, 0>",
-        "sddmm_coo_kernel<float, 4, 32, 1, 2, 32>", "sddmm_coo_kernel<float, 4, 32, 2, 2, 8>"]
+        "sddmm_coo_kernel<float, 4, 32, 1, 2, 32, 0, geot::SddmmParams>", "sddmm_coo_kernel<float, 4, 32, 2, 2, 8, 0, geot::SddmmParams>"]
 for w in want:
     for r in rows:
         if r[1].startswith(w):

@@ -14,8 +14,8 @@ WANT = [  # (object, demangled-name filter, what it is)
     ("inst_f32_0.o", "segment_reduce_kernel<float, 4, 32, 2, 0, 0, 35>", "gather_scatter F=256 fp32 (products gs256)"),
     ("inst_bf16_0.o", "segment_reduce_kernel<__nv_bfloat16, 8, 32, 1, 0, 2, 163>", "mh_spmm 8x32 bf16 (arxiv): lean ring with per-head weights"),
     ("inst_f32_0.o", "segment_fixup_kernel<float, 0>", "fixup pass (programmatic dependent launch)"),
-    ("sddmm.o", "sddmm_coo_kernel<float, 4, 32, 1, 2, 32>", "SDDMM F=128 fp32 (backward of gather_weight_scatter)"),
-    ("sddmm.o", "sddmm_coo_kernel<float, 4, 32, 2, 2, 8>", "SDDMM 8 heads x 32 fp32 (weight gradient of mh_spmm, arxiv)"),
+    ("sddmm.o", "sddmm_coo_kernel<float, 4, 32, 1, 2, 32, 0, geot::SddmmParams>", "SDDMM F=128 fp32 (backward of gather_weight_scatter)"),
+    ("sddmm.o", "sddmm_coo_kernel<float, 4, 32, 2, 2, 8, 0, geot::SddmmParams>", "SDDMM 8 heads x 32 fp32 (weight gradient of mh_spmm, arxiv)"),
     ("exchange.o", "push_rows_kernel<uint4>", "push transport: rows into the peers' symmetric memory"),
     ("abi.o", "scatter_add_kernel<float4>", "index_scatter(sorted=False) fp32 sum: vector atomics"),
 ]
