@@ -3,7 +3,8 @@
 Same Python surface as the reference package (``/root/reference/geot/__init__.py:4-9``) for the hot
 path: ``index_scatter``, ``gather_scatter``, ``gather_weight_scatter``, ``mh_spmm``,
 ``mh_spmm_transposed``, ``csr_gws``, ``coo_to_csr``; plus ``segment_softmax`` (attention weights over the edges of each
-dst row, ``gnn.GATConv``), ``gatv2_score`` (the fused GATv2 attention score, ``gnn.GATv2Conv``), ``format_preprocess`` (segment pointers + edge-count partition) and
+dst row, ``gnn.GATConv``), ``gatv2_score`` (the fused GATv2 attention score, ``gnn.GATv2Conv``), ``graph_attention``
+(fused dot-product attention, ``gnn.TransformerConv``), ``format_preprocess`` (segment pointers + edge-count partition) and
 ``dist`` (dst-row sharding over the GPUs of one box).  The operators are ``torch.ops.geot.*``
 registered by ``geot_b200/_C.so`` (thin bindings over the C ABI in ``include/geot_b200.h``).
 
@@ -38,6 +39,7 @@ from .gather_weight_scatter import gather_weight_scatter  # noqa: E402
 from .mh_spmm import mh_spmm, mh_spmm_transposed  # noqa: E402
 from .softmax import segment_softmax  # noqa: E402
 from .gatv2 import gatv2_score  # noqa: E402
+from .attention import graph_attention  # noqa: E402
 from .gather_weight_scatter import sddmm_coo_impl  # noqa: E402
 from .csr_gws import csr_gws, coo_to_csr  # noqa: E402
 from .format_preprocess import format_preprocess, Plan, clear_plan_cache  # noqa: E402
@@ -47,4 +49,4 @@ from . import dist  # noqa: E402
 
 __all__ = ["index_scatter", "gather_scatter", "gather_weight_scatter", "mh_spmm", "mh_spmm_transposed", "csr_gws",
            "coo_to_csr", "sddmm_coo_impl", "pattern_transform", "format_preprocess", "Plan", "clear_plan_cache", "dist",
-           "segment_softmax", "gatv2_score"]
+           "segment_softmax", "gatv2_score", "graph_attention"]

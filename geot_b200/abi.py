@@ -31,6 +31,8 @@ SYMBOLS = [
     "geot_b200_src_blocks_scratch_bytes", "geot_b200_src_blocks_build", "geot_b200_src_blocks_workspace_bytes",
     "geot_b200_segment_softmax_workspace_bytes", "geot_b200_segment_softmax", "geot_b200_segment_softmax_backward",
     "geot_b200_gatv2_score", "geot_b200_gatv2_grad_workspace_bytes", "geot_b200_gatv2_grad",
+    "geot_b200_graph_attention_workspace_bytes", "geot_b200_graph_attention",
+    "geot_b200_graph_attention_grad_workspace_bytes", "geot_b200_graph_attention_grad",
 ]
 
 
@@ -112,6 +114,15 @@ def lib() -> ctypes.CDLL:
         L.geot_b200_gatv2_grad_workspace_bytes.argtypes = [i64, i64, i64, ci]
         L.geot_b200_gatv2_grad.argtypes = [vp, vp, vp, vp, vp, vp, ctypes.POINTER(GeotPlan), i64, vp, vp, i64, i64, i64,
                                            ci, ctypes.POINTER(ctypes.c_double), vp, sz, vp]
+        dp = ctypes.POINTER(ctypes.c_double)
+        L.geot_b200_graph_attention_workspace_bytes.restype = sz
+        L.geot_b200_graph_attention_workspace_bytes.argtypes = [i64, i64, i64, ci]
+        L.geot_b200_graph_attention.argtypes = [vp, vp, vp, vp, vp, ctypes.POINTER(GeotPlan), i64, vp, vp, i64, i64, i64,
+                                                ci, dp, vp, sz, vp]
+        L.geot_b200_graph_attention_grad_workspace_bytes.restype = sz
+        L.geot_b200_graph_attention_grad_workspace_bytes.argtypes = [i64, i64, i64, ci]
+        L.geot_b200_graph_attention_grad.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, ctypes.POINTER(GeotPlan), i64, vp, vp,
+                                                     vp, i64, i64, i64, ci, dp, vp, sz, vp]
         L.geot_b200_csr_to_coo.argtypes = [vp, ci, i64, i64, vp, vp]
         L.geot_b200_permute_edges.argtypes = [vp, vp, vp, i64, i64, vp]
         L.geot_b200_segment_reduce_host.argtypes = [vp, i64, vp, vp, vp, vp, i64, i64, i64, i64, ci, ci, ci]
@@ -323,6 +334,40 @@ def gatv2_grad(x_row, x_gat, att, grad_score, row_index, gat_index, S_out, negat
                                      ctypes.byref(ctypes.c_double(negative_slope)),
                                      _ptr(ws), n, _stream()), "gatv2_grad")
     return grad_row, grad_att
+
+
+def graph_attention(q, k, v, src_index, dst_index, scale, N_dst=None, plan: DevicePlan = None):
+    """(out [N_dst, H, F], lse [N_dst, H]) of the fused dot-product attention through geot_b200_graph_attention; q
+    [N_dst, H, F], k / v [N_src, H, F], dst_index sorted."""
+    E, H, F = dst_index.numel(), q.shape[1], q.shape[2]
+    N_dst = q.shape[0] if N_dst is None else N_dst
+    plan = plan if plan is not None else DevicePlan(dst_index)
+    out = torch.empty(N_dst, H, F, dtype=q.dtype, device=q.device)
+    acc = torch.float64 if q.dtype == torch.float64 else torch.float32
+    lse = torch.empty(N_dst, H, dtype=acc, device=q.device)
+    n = lib().geot_b200_graph_attention_workspace_bytes(E, H, F, DTYPE[q.dtype])
+    ws = torch.empty(n, dtype=torch.uint8, device=q.device)
+    check(lib().geot_b200_graph_attention(_ptr(q), _ptr(k), _ptr(v), _ptr(src_index), _ptr(dst_index), ctypes.byref(plan.c),
+                                          N_dst, _ptr(out), _ptr(lse), E, H, F, DTYPE[q.dtype],
+                                          ctypes.byref(ctypes.c_double(scale)), _ptr(ws), n, _stream()), "graph_attention")
+    return out, lse
+
+
+def graph_attention_grad(q, k, v, out, lse, grad_out, src_index, dst_index, scale, plan: DevicePlan = None):
+    """(grad_q, p [E, H], scale * ds [E, H]) of the dst pass of the backward through geot_b200_graph_attention_grad."""
+    E, H, F = dst_index.numel(), q.shape[1], q.shape[2]
+    plan = plan if plan is not None else DevicePlan(dst_index)
+    grad_q = torch.empty_like(q)
+    p = torch.empty(E, H, dtype=q.dtype, device=q.device)
+    ds = torch.empty(E, H, dtype=q.dtype, device=q.device)
+    n = lib().geot_b200_graph_attention_grad_workspace_bytes(E, H, F, DTYPE[q.dtype])
+    ws = torch.empty(n, dtype=torch.uint8, device=q.device)
+    check(lib().geot_b200_graph_attention_grad(_ptr(q), _ptr(k), _ptr(v), _ptr(out), _ptr(lse), _ptr(grad_out),
+                                               _ptr(src_index), _ptr(dst_index), ctypes.byref(plan.c), q.shape[0],
+                                               _ptr(grad_q), _ptr(p), _ptr(ds), E, H, F, DTYPE[q.dtype],
+                                               ctypes.byref(ctypes.c_double(scale)), _ptr(ws), n, _stream()),
+          "graph_attention_grad")
+    return grad_q, p, ds
 
 
 def csr_to_coo(rowptr, E):

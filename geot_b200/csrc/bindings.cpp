@@ -20,6 +20,7 @@
 
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 #include <list>
 #include <mutex>
 #include <string>
@@ -579,6 +580,95 @@ std::tuple<at::Tensor, at::Tensor, at::Tensor> gatv2_score_backward_impl(
   return std::make_tuple(gl, gr, ga);
 }
 
+// ---- dot-product graph attention ------------------------------------------------------------------------------------
+// geot::graph_attention -> (out [N_dst, H, F], lse [N_dst, H] fp32 / fp64): q [N_dst, H, F] by dst, k / v [N_src, H, F]
+// by src, dst_index sorted (the plan cache says so; an unsorted index is refused), N_dst = q.size(0).
+void check_attention_operands(const at::Tensor &q, const at::Tensor &k, const at::Tensor &v, const at::Tensor &src_index,
+                              const at::Tensor &dst_index, const char *what) {
+  TORCH_CHECK(q.is_cuda() && k.is_cuda() && v.is_cuda(), "geot::", what,
+              ": q, k and v must be CUDA tensors (this build has no CPU path)");
+  check_index(src_index, "src_index");
+  check_index(dst_index, "dst_index");
+  TORCH_CHECK(src_index.dim() == 1 && dst_index.dim() == 1 && src_index.numel() == dst_index.numel(), "geot::", what,
+              ": src_index and dst_index must be 1 dimensional and of the same length");
+  TORCH_CHECK(q.dim() == 3 && k.dim() == 3 && v.dim() == 3 && k.sizes() == v.sizes() && q.size(1) == k.size(1) &&
+                  q.size(2) == k.size(2),
+              "geot::", what, ": q must be [N_dst, H, F] and k, v [N_src, H, F] with the same H and F");
+  TORCH_CHECK(q.size(1) > 0 && q.size(2) > 0, "geot::", what, ": q, k and v must have at least one head and one feature");
+  TORCH_CHECK(k.scalar_type() == q.scalar_type() && v.scalar_type() == q.scalar_type(), "geot::", what,
+              ": q, k and v must have the same dtype");
+  const auto dev = q.device();
+  TORCH_CHECK(k.device() == dev && v.device() == dev && src_index.device() == dev && dst_index.device() == dev, "geot::",
+              what, ": all operands must be on the same device");
+}
+
+at::ScalarType lse_type(const at::Tensor &q) { return q.scalar_type() == at::kDouble ? at::kDouble : at::kFloat; }
+
+std::tuple<at::Tensor, at::Tensor> graph_attention_impl(at::Tensor q, at::Tensor k, at::Tensor v, at::Tensor src_index,
+                                                        at::Tensor dst_index, double scale) {
+  check_attention_operands(q, k, v, src_index, dst_index, "graph_attention");
+  const int dtype = dtype_enum(q);
+  c10::cuda::CUDAGuard guard(q.device());
+  const at::Tensor qc = q.contiguous(), kc = k.contiguous(), vc = v.contiguous();
+  const at::Tensor si = src_index.contiguous(), di = dst_index.contiguous();
+  const int64_t E = di.numel(), N = qc.size(0), H = qc.size(1), F = qc.size(2);
+  at::Tensor out = at::empty_like(qc);
+  at::Tensor lse = at::empty({N, H}, qc.options().dtype(lse_type(qc)));
+  if (E == 0) {            // no edge: every row is empty
+    out.zero_();
+    lse.fill_(-std::numeric_limits<double>::infinity());
+    return std::make_tuple(out, lse);
+  }
+  at::Tensor plan_buf;
+  const geot_plan_t plan = softmax_plan(di, "graph_attention", &plan_buf);
+  TORCH_CHECK(plan.max_row < N, "geot::graph_attention: dst_index holds ", plan.max_row, " but q has ", N, " rows");
+  const size_t ws_bytes = geot_b200_graph_attention_workspace_bytes(E, H, F, dtype);
+  at::Tensor ws = at::empty({(int64_t)ws_bytes}, qc.options().dtype(at::kByte));
+  check_status(geot_b200_graph_attention(qc.data_ptr(), kc.data_ptr(), vc.data_ptr(), si.data_ptr<int64_t>(),
+                                         di.data_ptr<int64_t>(), &plan, N, out.data_ptr(), lse.data_ptr(), E, H, F, dtype,
+                                         &scale, ws.data_ptr(), ws_bytes, at::cuda::getCurrentCUDAStream()),
+               "graph_attention");
+  return std::make_tuple(out, lse);
+}
+
+// geot::graph_attention_backward -> (grad_q [N_dst, H, F], p [E, H], ds [E, H]): the dst pass of the backward; ds is
+// scale * d loss / d score.  grad_k and grad_v are mh_spmm passes on the transposed edge list (attention.py).
+std::tuple<at::Tensor, at::Tensor, at::Tensor> graph_attention_backward_impl(
+    at::Tensor grad, at::Tensor q, at::Tensor k, at::Tensor v, at::Tensor out, at::Tensor lse, at::Tensor src_index,
+    at::Tensor dst_index, double scale) {
+  check_attention_operands(q, k, v, src_index, dst_index, "graph_attention_backward");
+  TORCH_CHECK(grad.sizes() == q.sizes() && out.sizes() == q.sizes(),
+              "geot::graph_attention_backward: grad and out must have the shape of q");
+  TORCH_CHECK(grad.scalar_type() == q.scalar_type() && out.scalar_type() == q.scalar_type() && grad.device() == q.device() &&
+                  out.device() == q.device(),
+              "geot::graph_attention_backward: grad and out must have the dtype and device of q");
+  TORCH_CHECK(lse.dim() == 2 && lse.size(0) == q.size(0) && lse.size(1) == q.size(1) && lse.scalar_type() == lse_type(q) &&
+                  lse.device() == q.device(),
+              "geot::graph_attention_backward: lse must be [N_dst, H] in the accumulator type");
+  const int dtype = dtype_enum(q);
+  c10::cuda::CUDAGuard guard(q.device());
+  const at::Tensor qc = q.contiguous(), kc = k.contiguous(), vc = v.contiguous(), oc = out.contiguous(),
+                   lc = lse.contiguous(), g = grad.contiguous();
+  const at::Tensor si = src_index.contiguous(), di = dst_index.contiguous();
+  const int64_t E = di.numel(), N = qc.size(0), H = qc.size(1), F = qc.size(2);
+  at::Tensor grad_q = at::empty_like(qc);
+  at::Tensor p = at::empty({E, H}, qc.options()), ds = at::empty({E, H}, qc.options());
+  if (E == 0) {
+    grad_q.zero_();
+    return std::make_tuple(grad_q, p, ds);
+  }
+  at::Tensor plan_buf;
+  const geot_plan_t plan = softmax_plan(di, "graph_attention_backward", &plan_buf);
+  const size_t ws_bytes = geot_b200_graph_attention_grad_workspace_bytes(E, H, F, dtype);
+  at::Tensor ws = at::empty({(int64_t)ws_bytes}, qc.options().dtype(at::kByte));
+  check_status(geot_b200_graph_attention_grad(qc.data_ptr(), kc.data_ptr(), vc.data_ptr(), oc.data_ptr(), lc.data_ptr(),
+                                              g.data_ptr(), si.data_ptr<int64_t>(), di.data_ptr<int64_t>(), &plan, N,
+                                              grad_q.data_ptr(), p.data_ptr(), ds.data_ptr(), E, H, F, dtype, &scale,
+                                              ws.data_ptr(), ws_bytes, at::cuda::getCurrentCUDAStream()),
+               "graph_attention_backward");
+  return std::make_tuple(grad_q, p, ds);
+}
+
 // ---- CSR entry point ------------------------------------------------------------------------------------
 // Cache of the COO row index expanded from a CSR row pointer, keyed like the plans (storage + version).
 struct CsrEntry {
@@ -686,6 +776,9 @@ TORCH_LIBRARY_FRAGMENT(geot, m) {
   m.def("gatv2_score_backward(Tensor grad, Tensor x_l, Tensor x_r, Tensor att, Tensor src_index, Tensor dst_index, "
         "Tensor t_perm, Tensor t_dst_index, Tensor t_src_index, float negative_slope, bool need_x_l, bool need_x_r, "
         "bool need_att) -> (Tensor, Tensor, Tensor)");
+  m.def("graph_attention(Tensor q, Tensor k, Tensor v, Tensor src_index, Tensor dst_index, float scale) -> (Tensor, Tensor)");
+  m.def("graph_attention_backward(Tensor grad, Tensor q, Tensor k, Tensor v, Tensor out, Tensor lse, Tensor src_index, "
+        "Tensor dst_index, float scale) -> (Tensor, Tensor, Tensor)");
   m.def("clear_plan_cache() -> ()", []() { clear_plan_cache(); });
   m.def("abi_version() -> int", []() { return (int64_t)geot_b200_version(); });
 }
@@ -707,4 +800,6 @@ TORCH_LIBRARY_IMPL(geot, CUDA, m) {
   m.impl("segment_softmax_backward", segment_softmax_backward_impl);
   m.impl("gatv2_score", gatv2_score_impl);
   m.impl("gatv2_score_backward", gatv2_score_backward_impl);
+  m.impl("graph_attention", graph_attention_impl);
+  m.impl("graph_attention_backward", graph_attention_backward_impl);
 }

@@ -77,6 +77,18 @@ def _(grad, x_l, x_r, att, src_index, dst_index, t_perm, t_dst_index, t_src_inde
     return like(x_l, need_x_l), like(x_r, need_x_r), like(att, need_att)
 
 
+@torch.library.register_fake("geot::graph_attention")
+def _(q, k, v, src_index, dst_index, scale):
+    acc = torch.float64 if q.dtype == torch.float64 else torch.float32
+    return q.new_empty(q.shape), q.new_empty([q.shape[0], q.shape[1]], dtype=acc)
+
+
+@torch.library.register_fake("geot::graph_attention_backward")
+def _(grad, q, k, v, out, lse, src_index, dst_index, scale):
+    E, H = dst_index.shape[0], q.shape[1]
+    return q.new_empty(q.shape), q.new_empty([E, H]), q.new_empty([E, H])
+
+
 @torch.library.register_fake("geot::csr_gws_impl")
 def _(indptr, indices, weight, src):
     return src.new_empty([indptr.shape[0], src.shape[1]])

@@ -15,6 +15,8 @@ PyG / torch_sparse are not part of this build, so the same math is restated on p
   aggregation ``mh_spmm`` -- both deterministic kernels of this library, both differentiable.
 * GATv2 layer (PyG ``GATv2Conv``, ``share_weights=False``, without dropout and edge features): the attention score is
   the fused ``gatv2_score``, then ``segment_softmax`` and ``mh_spmm``.
+* Transformer layer (PyG ``TransformerConv`` without ``beta``, edge features and dropout): the fused
+  ``graph_attention`` (dot-product scores, softmax and aggregation in one pass), then the skip connection.
 * Stack (``models/basicgnn.py:216-264``): ``conv -> ReLU`` for every layer but the last; dropout p = 0.
 
 The dense ``lin`` layers are cuBLAS GEMMs through ``torch.nn.Linear`` (library code, not part of the hot
@@ -32,6 +34,7 @@ from .gather_weight_scatter import gather_weight_scatter
 from .mh_spmm import mh_spmm
 from .softmax import segment_softmax
 from .gatv2 import gatv2_score
+from .attention import graph_attention
 
 
 def add_self_loops(src_index: torch.Tensor, dst_index: torch.Tensor, num_nodes: int,
@@ -166,6 +169,36 @@ class GATv2Conv(nn.Module):
         out = _pad_rows(mh_spmm(src_index, dst_index, alpha, x_l), N)
         out = out.reshape(N, H * F) if self.concat else out.mean(1)
         return out + self.bias if self.bias is not None else out
+
+
+class TransformerConv(nn.Module):
+    """PyG's ``TransformerConv`` math on a dst-sorted edge list (no self loops are added, as in PyG):
+    ``q = lin_query(x)``, ``k = lin_key(x)``, ``v = lin_value(x)`` as ``[N, H, F]``; per edge and head
+    ``alpha = softmax_row(<q[dst], k[src]> / sqrt(F))`` and ``out[dst] = sum alpha * v[src]`` (the fused
+    ``graph_attention``, which materialises no ``[E, H]`` tensor); the heads are concatenated (``concat``) or averaged,
+    then ``lin_skip(x)`` is added when ``root_weight`` is set.  ``lin_query``, ``lin_key`` and ``lin_value`` map to
+    ``H * F`` and ``lin_skip`` to ``H * F`` (``concat``) or ``F``, all with a bias when ``bias`` is set and torch's default
+    initialisation, as PyG's ``Linear``.  Left out of PyG's options: ``beta`` (the gated skip), ``edge_dim`` (edge
+    features) and attention ``dropout``; one node set (no bipartite input).  Differentiable end to end."""
+
+    def __init__(self, in_channels: int, out_channels: int, heads: int = 1, concat: bool = True, bias: bool = True,
+                 root_weight: bool = True):
+        super().__init__()
+        self.heads, self.out_channels, self.concat, self.root_weight = heads, out_channels, concat, root_weight
+        self.lin_query = nn.Linear(in_channels, heads * out_channels, bias=bias)
+        self.lin_key = nn.Linear(in_channels, heads * out_channels, bias=bias)
+        self.lin_value = nn.Linear(in_channels, heads * out_channels, bias=bias)
+        self.lin_skip = (nn.Linear(in_channels, heads * out_channels if concat else out_channels, bias=bias)
+                         if root_weight else None)
+
+    def forward(self, x, src_index, dst_index):
+        N, H, F = x.shape[0], self.heads, self.out_channels
+        q = self.lin_query(x).view(N, H, F)
+        k = self.lin_key(x).view(N, H, F)
+        v = self.lin_value(x).view(N, H, F)
+        out = graph_attention(q, k, v, src_index, dst_index)
+        out = out.reshape(N, H * F) if self.concat else out.mean(1)
+        return out + self.lin_skip(x) if self.lin_skip is not None else out
 
 
 class _Stack(nn.Module):

@@ -34,6 +34,29 @@ def mh_spmm_transposed(src_index: torch.Tensor, dst_index: torch.Tensor, weight:
     return torch.ops.geot.mh_spmm(src_index, dst_index, weight, src, reduce)
 
 
+def src_side_spmm(src_index: torch.Tensor, dst_index: torch.Tensor, weight: torch.Tensor, x: torch.Tensor,
+                  n_rows: int, head_major: bool = False) -> torch.Tensor:
+    """``out[j, h, :] = sum_{e : src_index[e] = j} weight[e, h] * x[dst_index[e], h, :]``, ``[n_rows, H, F]``: the
+    forward kernel on the cached transposed (src-sorted) edge list, with the weights (``[E, H]``, or ``[H, E]`` with
+    ``head_major``) carried into that edge order by ``geot_b200_permute_edges``.  Rows past the largest src index are
+    zero.  The src-side gradients of ``mh_spmm`` and of ``graph_attention``."""
+    from . import abi
+    from .transpose import transposed_edges
+    t = transposed_edges(src_index, dst_index)
+    w = weight.contiguous()
+    with torch.cuda.device(w.device):
+        if head_major:
+            w_perm = torch.empty_like(w)
+            for h in range(w.shape[0]):
+                abi.permute_edges(w[h], t.perm, out=w_perm[h])
+        else:
+            w_perm = abi.permute_edges(w, t.perm)
+    g = torch.ops.geot.mh_spmm(t.src_index, t.dst_index, w_perm, x, "sum")
+    if g.shape[0] < n_rows:      # trailing src rows that no edge reads
+        g = torch.cat([g, g.new_zeros((n_rows - g.shape[0],) + tuple(g.shape[1:]))], 0)
+    return g
+
+
 def _setup_context(ctx, inputs, output):
     src_index, dst_index, weight, src, reduce = inputs
     ctx.save_for_backward(src_index, dst_index, weight, src)
@@ -41,8 +64,6 @@ def _setup_context(ctx, inputs, output):
 
 
 def _backward(ctx, grad):
-    from . import abi
-    from .transpose import transposed_edges
     src_index, dst_index, weight, src = ctx.saved_tensors
     if ctx.reduce not in ("sum", "mean"):
         raise NotImplementedError("geot.mh_spmm: no backward for reduce=%r (sum and mean only: the others need the "
@@ -57,19 +78,7 @@ def _backward(ctx, grad):
         grad = (grad * scale.view(-1, 1, 1)).to(grad.dtype)
     weight_grad = src_grad = None
     if ctx.needs_input_grad[3]:
-        t = transposed_edges(src_index, dst_index)
-        w = weight.contiguous()
-        with torch.cuda.device(w.device):
-            if head_major:
-                w_perm = torch.empty_like(w)
-                for h in range(H):
-                    abi.permute_edges(w[h], t.perm, out=w_perm[h])
-            else:
-                w_perm = abi.permute_edges(w, t.perm)
-        g = torch.ops.geot.mh_spmm(t.src_index, t.dst_index, w_perm, grad, "sum")
-        if g.shape[0] < src.shape[0]:      # trailing src rows that no edge reads
-            g = torch.cat([g, g.new_zeros((src.shape[0] - g.shape[0],) + tuple(g.shape[1:]))], 0)
-        src_grad = g
+        src_grad = src_side_spmm(src_index, dst_index, weight, grad, src.shape[0], head_major)
     if ctx.needs_input_grad[2]:
         # dst-sorted edge order: the kernel keeps the grad row in registers across a segment
         weight_grad = torch.ops.geot.sddmm_mh_impl(src_index, dst_index, grad, src, head_major)

@@ -277,6 +277,39 @@ GEOT_API int geot_b200_gatv2_grad(const void *x_row, const void *x_gat, const vo
                          void *grad_row, void *grad_att, int64_t E, int64_t H, int64_t F, int dtype,
                          const double *negative_slope, void *workspace, size_t workspace_bytes, cudaStream_t stream);
 
+/* Dot-product graph attention, fused (PyG TransformerConv's attention, without beta, edge features or dropout):
+ *     score[e, h]  = scale * < q[dst_index[e], h, :], k[src_index[e], h, :] >          scale = *scale (host memory)
+ *     out[i, h, :] = sum_{e : dst_index[e] = i} alpha[e, h] * v[src_index[e], h, :],   alpha = softmax of score over row i
+ *     lse[i, h]    = log sum_{e : dst_index[e] = i} exp(score[e, h])
+ * q [N_dst, H, F], k / v [N_src, H, F], out [N_dst, H, F] of `dtype`; lse [N_dst, H] in the accumulator type (fp32, or
+ * fp64 for fp64).  One edge-balanced pass with an online softmax: no [E, H] score or alpha is stored.  dst_index is
+ * non-decreasing: plan is its plan (geot_b200_format_preprocess) with plan->max_row < N_dst.  Every row of out and lse
+ * is written; rows without edges get out = 0 and lse = -inf.  bf16/fp16/fp32 accumulate in fp32, fp64 in fp64, with the
+ * accurate exp / log and IEEE division, one rounding on every store; a NaN score makes its row NaN.  No atomics: the
+ * result is bit-reproducible.  A launch covers whole heads of at most 256 columns (128 for fp64): a head wider than that
+ * returns GEOT_ERR_UNSUPPORTED.  Returns GEOT_ERR_EMPTY for E == 0, GEOT_ERR_INVALID_ARG for an unsorted plan, a plan of
+ * another index or a plan whose largest index is >= N_dst; workspace: geot_b200_graph_attention_workspace_bytes
+ * (256-byte aligned). */
+GEOT_API size_t geot_b200_graph_attention_workspace_bytes(int64_t E, int64_t H, int64_t F, int dtype);
+GEOT_API int geot_b200_graph_attention(const void *q, const void *k, const void *v, const int64_t *src_index,
+                              const int64_t *dst_index, const geot_plan_t *plan, int64_t N_dst, void *out, void *lse,
+                              int64_t E, int64_t H, int64_t F, int dtype, const double *scale, void *workspace,
+                              size_t workspace_bytes, cudaStream_t stream);
+/* The dst pass of its backward, recomputing alpha from lse (FlashAttention-2).  With g = grad_out [N_dst, H, F]:
+ *     D[i, h] = < g[i, h], out[i, h] >,   p[e, h] = exp(score[e, h] - lse[dst, h]),
+ *     ds[e, h] = scale * p[e, h] * (< g[dst, h], v[src, h] > - D[dst, h]),
+ *     grad_q[i] = sum_{e : dst_index[e] = i} ds[e, h] * k[src, h, :]
+ * grad_q [N_dst, H, F] is fully written (rows without edges are 0); p and ds [E, H] (`dtype`) are the weights of the
+ * src-side gradients grad_k = sum_{e : src = j} ds q[dst] and grad_v = sum_{e : src = j} p g[dst], which
+ * geot_b200_mh_spmm computes on the transposed edge list.  Same operands, precision, determinism and status codes as
+ * the forward; workspace: geot_b200_graph_attention_grad_workspace_bytes (256-byte aligned). */
+GEOT_API size_t geot_b200_graph_attention_grad_workspace_bytes(int64_t E, int64_t H, int64_t F, int dtype);
+GEOT_API int geot_b200_graph_attention_grad(const void *q, const void *k, const void *v, const void *out,
+                                   const void *lse, const void *grad_out, const int64_t *src_index,
+                                   const int64_t *dst_index, const geot_plan_t *plan, int64_t N_dst, void *grad_q,
+                                   void *p, void *ds, int64_t E, int64_t H, int64_t F, int dtype, const double *scale,
+                                   void *workspace, size_t workspace_bytes, cudaStream_t stream);
+
 /* CSR row pointer -> sorted COO row index (the inverse of geot::coo_to_csr): row_index[e] = r for
  * rowptr[r] <= e < rowptr[r+1].  rowptr has S+1 entries of 32 or 64 bits (rowptr_bits).  Lets the CSR entry
  * point csr_gws (csrc/csr_gws.cpp:24-35, csr_gws_cuda.cu) run on the same kernels. */
